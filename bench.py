@@ -6,6 +6,7 @@ random-init weights, policy-P0 bit assignment derived from the reference's delta
     python bench.py --gpus 1 --steps 20 --warmup 5
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference's own path on the host CPU cores
+    python bench.py ... --dump-outputs DIR    # also writes the last timed step's logits to DIR/logits.npy
 
 A "step" is one forward pass of one batch (256 images per GPU) through the whole hot path:
 stem -> 52 quantised/fp32-weight convs on tcgen05 (fused dequant+BN+residual+ReLU epilogues)
@@ -25,6 +26,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "semilayer-wise-mixed-precision-quantization_b200")
 sys.path.insert(0, PKG)
+DUMP_LIMIT_BYTES = 64 << 20
 
 METRIC = "ResNet-50 mixed 8/4-bit images/s"
 
@@ -224,6 +226,18 @@ def bind_to_gpu_numa_node(local):
         return {"bound": False, "why": "%s: %s" % (type(e).__name__, e)}
 
 
+def dump_logits(out_dir, logits, rank, world):
+    """Writes one rank's logits [batch, classes] as float32 .npy.  The files of all ranks together stay under
+    DUMP_LIMIT_BYTES: past that, a fixed seeded sample of the rows (the same rows on every run) is written."""
+    import numpy as np
+    cap = max(1, DUMP_LIMIT_BYTES // world // (4 * logits.shape[1]))
+    if logits.shape[0] > cap:
+        logits = logits[np.sort(np.random.default_rng(0).choice(logits.shape[0], cap, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    name = "logits.npy" if world == 1 else "logits_rank%d.npy" % rank
+    np.save(os.path.join(out_dir, name), np.ascontiguousarray(logits, dtype=np.float32))
+
+
 def measure_i8_peak(lib, L, st, torch):
     """Dense kind::i8 tensor rate of THIS GPU (slq_probe_i8_peak: every SM streams M128 x N256 x K32 MMAs):
     burst = best of 5 launches of ~20 ms; sustained = one >= 2 s train of launches."""
@@ -268,7 +282,14 @@ def main():
                     help="A/B: resident-weight layers take u8 weight tiles through TMA instead of packed codes unpacked in smem")
     ap.add_argument("--no-fuse-tail", action="store_true",
                     help="A/B: downsample conv and conv3 of a stage's first block as two launches (identity through HBM)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the logits of the last timed step to DIR/logits.npy (float32; "
+                         "logits_rank<r>.npy per rank with several GPUs) to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -414,6 +435,8 @@ def main():
     e1.record(st)
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs:  # before the e2e loops below overwrite the engine's logits buffer
+        dump_logits(args.dump_outputs, eng.logits.cpu().numpy(), rank, world)
     ms = e0.elapsed_time(e1)
     tmax = torch.tensor([ms], device=dev)
     if world > 1:
@@ -425,7 +448,9 @@ def main():
     # The loader-side pattern of the reference (functions.py:110-113: inputs.to(device); net(inputs))
     # with pinned memory and a copy stream: batch i+1 crosses PCIe while batch i computes; every
     # step's logits come back to the host (a blocking read), so nothing is deferred past the region.
-    e2e_steps = max(3, min(args.steps, 20))
+    # as many steps as the headline loop (--steps); with only one or two, the figure is mostly the time to fill
+    # the copy pipeline
+    e2e_steps = args.steps
     copy_stream = torch.cuda.Stream(dev)
     NB = 3  # input buffers: the copy engine always has the next batch queued behind the one in flight
     dbuf = [torch.empty_like(x) for _ in range(NB)]

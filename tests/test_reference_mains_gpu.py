@@ -14,11 +14,19 @@ bit / phase-flag / accuracy rows, the cumulative reduced-parameter total, per ph
 (layer number, channel count, parameter increment), and -- with the divide flavour pinned to the CPU one
 (SURVEY.md F5) -- every final conv weight, bit for bit.  The ORDER of the semilayers inside a phase comes
 from the KL/param ranking of the sweep, which this path perturbs by its u8 activation quantisation (the
-reference never quantises activations, F2): it is reported (rank correlation), not asserted."""
+reference never quantises activations, F2): it is reported (rank correlation), not asserted.
+
+The driver script is the reference project's, not this repository's, so that test runs only where the
+reference has been staged (oracle/make_ref.py).  The fixture alone pins the part of its outcome that needs no
+driver: the package's evaluation on the fixture's seeded batches gives the accuracy row, so every semilayer is
+accepted, every channel goes 8 -> 6 -> 4 bit, and the final weights are that progressive re-quantisation of the
+seeded model through the package's drop-in quantizer."""
 import os
+from collections import Counter
 
 import numpy as np
 import pytest
+import torch
 
 from helpers import GOLD
 
@@ -36,7 +44,10 @@ def _phases(rows):
 
 
 def test_unmodified_resnet50_main_against_the_package(monkeypatch):
+    import make_ref
     import run_main
+    if not make_ref.staged():
+        pytest.skip("the reference's resnet50_main.py is not staged under oracle/_ref")
     gold = np.load(os.path.join(GOLD, "main_resnet50.npz"))
     want = [r.split("\x1f") for r in gold["rows"]]
     b, n, hw, lseed, mseed = [int(v) for v in gold["config"]]
@@ -58,6 +69,49 @@ def test_unmodified_resnet50_main_against_the_package(monkeypatch):
     print("8-bit phase: %d of %d steps visit the same layer as the reference run" % (same_pos, len(w8)))
     kl = np.array([float(v) for v in got[2]])
     print("KL row, first steps: ours %s reference %s" % (kl[1:4], [float(v) for v in want[2][1:4]]))
+
+
+def test_resnet50_main_fixture_weights_from_the_package_quantizer(monkeypatch):
+    """The reference run of the fixture accepts every semilayer (the accuracy on its seeded batches never drops
+    below the fp32 model's) and so visits every channel of the 48 quantised convs once per phase, at 8, then 6,
+    then 4 bit.  On the package, the seeded model re-quantised that way with ``channel_wise_quantizationperchan``
+    on the GPU must be evaluated (``evaluate_acc_loss_softmax``) to the fixture's accuracy row after every phase,
+    and must end with the reference run's final conv weights bit for bit."""
+    import functions
+    import imagenet
+    import resnet
+    import run_main
+    gold = np.load(os.path.join(GOLD, "main_resnet50.npz"))
+    rows = [r.split("\x1f") for r in gold["rows"]]
+    b, n, hw, lseed, mseed = [int(v) for v in gold["config"]]
+    loader = imagenet.synthetic_loader(b, n, hw, seed=lseed)
+    monkeypatch.setenv("SLQ_DIV_MODE", "true")
+    torch.manual_seed(mseed)
+    net = resnet.resnet50(num_classes=1000).cuda()
+    convs = dict(functions.quantized_convs("resnet50", net))
+    preacc = functions.evaluate_acc_loss_softmax(net, "cuda", loader)[0]
+    params = [float(v) for v in rows[0]]
+    bits = [int(v) for v in rows[3][1:]]
+    assert len(params) == 280 and bits == sorted(bits, reverse=True) and sorted(set(bits)) == [4, 6, 8]
+    previous = {8: 32, 6: 8, 4: 6}
+    for bit in (8, 6, 4):
+        visited, accs = Counter(), set()
+        for i in range(1, len(params)):
+            if int(rows[3][i]) != bit:
+                continue
+            lnum, channels = int(rows[5][i]), int(rows[6][i])
+            K = convs[lnum].weight[0].numel()
+            assert params[i] - params[i - 1] == channels * K * (previous[bit] - bit) / 32  # the reference's layer map
+            visited[lnum] += channels
+            accs.add(float(rows[1][i]))
+        assert visited == {lnum: conv.out_channels for lnum, conv in convs.items()}
+        for conv in convs.values():
+            for c in range(conv.out_channels):
+                functions.channel_wise_quantizationperchan(conv.weight.data, bit, c)
+        acc = functions.evaluate_acc_loss_softmax(net, "cuda", loader)[0]
+        assert acc >= preacc and accs == {acc}, (bit, preacc, acc, accs)
+    assert params[-1] == 18092032.0
+    assert run_main.conv_weights_sha256(net) == str(gold["weights_sha256"])
 
 
 def test_reference_files_are_staged_unmodified():
