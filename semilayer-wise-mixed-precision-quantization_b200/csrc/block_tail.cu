@@ -31,6 +31,7 @@
 #include <new>
 
 #include "conv_common.cuh"
+#include "tma_host.cuh"
 #include "umma_ptx.cuh"
 
 struct slq_blocktail {
@@ -66,13 +67,6 @@ struct BtArgs {
             // store, 8 no downsample MMAs, 32 results overwritten (the arithmetic itself still runs: a runtime flag)
 };
 #define BT_DBG(a) (kDebugTrace ? (a).dbg : 0)
-// wait statistics of CTA 0 (debug build, slq_debug_set_trace with a buffer of >= 16 int64): cycles a role spent blocked
-__device__ __forceinline__ void bt_wait(uint32_t bar, uint32_t parity, long long *acc, bool on) {
-  if (!kDebugTrace || !on) { mbar_wait(bar, parity); return; }
-  const long long t0 = clock64();
-  mbar_wait(bar, parity);
-  *acc += clock64() - t0;
-}
 
 // per-channel constants of the fused epilogue, structure of arrays in shared memory (64 channels):
 //   A3 = wscale3 * s_y2 [* inv] ; Z3 = zf3 * A3 ; Ad = wscaled * s_x [* inv] ; Zd = zfd * Ad ; B = (bias3 + biasd) [* inv]
@@ -136,11 +130,7 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA3, const __grid_constan
     mbar_init(bfull_bar, 1);
     fence_barrier_init();
   }
-  if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                     smem_u32((const void *)tmem_slot)), "r"(512) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 2) tmem_alloc(tmem_slot, 512);
   // the ones groups behind the weight rows of every resident B tile (row 0 of the group = 0x01.., rows 1..15 = 0)
   for (int i = threadIdx.x; i < kb_tile * 16 * (SWZ / 16); i += blockDim.x) {
     const int t = i / (16 * (SWZ / 16)), rem = i % (16 * (SWZ / 16));
@@ -186,7 +176,7 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA3, const __grid_constan
       }
       for (int kb = 0; kb < kb_tile; ++kb, ++c) {
         const int s = c % a.stages;
-        bt_wait(empty_bar(p, s), (uint32_t)(((c / a.stages) & 1) ^ 1), &w_empty, st_on);
+        mbar_wait_stat(empty_bar(p, s), (uint32_t)(((c / a.stages) & 1) ^ 1), w_empty, st_on);
         if (elect_one()) {
           const uint32_t dst = smem_base + a.ring_off + (p * a.stages + s) * kABytes;
           mbar_expect_tx(full_bar(p, s), kABytes);
@@ -213,11 +203,11 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA3, const __grid_constan
     const bool st_on = kDebugTrace && a.stats != nullptr && blockIdx.x == 0;
     const long long t_begin = clock64();
     for (int i = p; i < count; i += 2, ++t) {
-      if (t >= 1) bt_wait(tempty_bar(p), (uint32_t)((t - 1) & 1), &w_tempty, st_on);  // the crew drained this pipeline's previous tile
+      if (t >= 1) mbar_wait_stat(tempty_bar(p), (uint32_t)((t - 1) & 1), w_tempty, st_on);  // the crew drained this pipeline's previous tile
       tc_fence_after();
       for (int kb = 0; kb < kb_tile; ++kb, ++c) {
         const int s = c % a.stages;
-        bt_wait(full_bar(p, s), (uint32_t)((c / a.stages) & 1), &w_full, st_on);
+        mbar_wait_stat(full_bar(p, s), (uint32_t)((c / a.stages) & 1), w_full, st_on);
         tc_fence_after();
         if (elect_one()) {
           const uint64_t da = make_smem_desc<SWZ>(smem_base + a.ring_off + (p * a.stages + s) * kABytes);
@@ -268,7 +258,7 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA3, const __grid_constan
       const long long m = (long long)m_tile * kTileM + row;
       const bool valid = m < a.M;
       const uint32_t tcol = tlane + p * kBtAccCols;
-      bt_wait(tfull_bar(p), (uint32_t)(t & 1), &w_tfull, st_on);
+      mbar_wait_stat(tfull_bar(p), (uint32_t)(t & 1), w_tfull, st_on);
       if (st_on) tseg = clock64();
       tc_fence_after();
       uint32_t a3[16], lo[16], hi[16];
@@ -363,7 +353,7 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA3, const __grid_constan
   __syncthreads();
   if (warp == 2) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
+    tmem_dealloc(tmem_base, 512);
   }
 }
 
@@ -408,71 +398,11 @@ __global__ void __launch_bounds__(128) block_tail_simt_kernel(BtArgs a, const ui
   else reinterpret_cast<float *>(a.out)[m * a.Cout + oc] = fmaxf(y, 0.f);
 }
 
-typedef CUresult (*BtEncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                    const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-typedef CUresult (*BtEncodeIm2colFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                     const cuuint64_t *, const int *, const int *, cuuint32_t, cuuint32_t,
-                                     const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                     CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static int bt_encoders(BtEncodeTiledFn *tiled, BtEncodeIm2colFn *im2col) {
-  static BtEncodeTiledFn f_tiled = nullptr;
-  static BtEncodeIm2colFn f_im2col = nullptr;
-  if (!f_tiled || !f_im2col) {
-    void *p = nullptr;
-    cudaDriverEntryPointQueryResult qr;
-    SLQ_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qr));
-    SLQ_CHECK_ARG(qr == cudaDriverEntryPointSuccess && p, "cuTensorMapEncodeTiled not available from the driver");
-    f_tiled = (BtEncodeTiledFn)p;
-    p = nullptr;
-    SLQ_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeIm2col", &p, cudaEnableDefault, &qr));
-    SLQ_CHECK_ARG(qr == cudaDriverEntryPointSuccess && p, "cuTensorMapEncodeIm2col not available from the driver");
-    f_im2col = (BtEncodeIm2colFn)p;
-  }
-  *tiled = f_tiled;
-  *im2col = f_im2col;
-  return SLQ_OK;
-}
-
-static int bt_tiled_u8(CUtensorMap *tm, const void *ptr, long long rows, int cols, int box_cols, int box_rows,
-                       CUtensorMapSwizzle sw, const char *what) {
-  BtEncodeTiledFn enc;
-  BtEncodeIm2colFn enc2;
-  int rc = bt_encoders(&enc, &enc2);
-  if (rc != SLQ_OK) return rc;
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)cols};
-  cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
-  cuuint32_t es[2] = {1, 1};
-  const CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void *>(ptr), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled(%s) failed: CUresult %d", what, (int)r);
-    return SLQ_ERR_CUDA;
-  }
-  return SLQ_OK;
-}
-
 template <int SWZ, int OUT>
 static int bt_launch(slq_blocktail *h, const BtArgs &a, cudaStream_t st) {
-  static bool attr_done[kMaxDevices] = {false};
-  const int dev = current_device();
-  if (dev >= kMaxDevices || !attr_done[dev]) {
-    SLQ_CUDA(cudaFuncSetAttribute(block_tail_kernel<SWZ, OUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-    if (dev < kMaxDevices) attr_done[dev] = true;
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)h->grid);
-  cfg.blockDim = dim3(kBtThreads);
-  cfg.dynamicSmemBytes = (size_t)h->smem_bytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  SLQ_CUDA(cudaLaunchKernelEx(&cfg, block_tail_kernel<SWZ, OUT>, h->tmA3, h->tmAd, h->tmB3, h->tmBd, h->tmO, a));
+  constexpr auto kernel = block_tail_kernel<SWZ, OUT>;
+  SLQ_CUDA(set_smem_limit_once<kernel>(232448));
+  SLQ_CUDA(launch_pdl(kernel, h->grid, kBtThreads, h->smem_bytes, st, h->tmA3, h->tmAd, h->tmB3, h->tmBd, h->tmO, a));
   return SLQ_OK;
 }
 
@@ -532,33 +462,15 @@ extern "C" int slq_blocktail_create(const slq_blocktail_desc *d, const uint8_t *
   h->grid = (int)(std::min<long long>(std::max(sm_count() / h->n_tiles, 1), m_tiles)) * h->n_tiles;
   if (d->impl == SLQ_IMPL_UMMA) {
     const CUtensorMapSwizzle sw = swz == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
-    int rc = bt_tiled_u8(&h->tmA3, y2, h->M, d->Cmid, swz, kTileM, sw, "y2");
-    if (rc == SLQ_OK) rc = bt_tiled_u8(&h->tmB3, wg3, d->Cout, d->Cmid, swz, 64, sw, "W3");
-    if (rc == SLQ_OK) rc = bt_tiled_u8(&h->tmBd, wgd, (long long)h->n_tiles * 128, d->Cin, swz, 128, sw, "Wd");
+    int rc = encode_tiled_u8(&h->tmA3, y2, h->M, d->Cmid, swz, kTileM, sw, "y2");
+    if (rc == SLQ_OK) rc = encode_tiled_u8(&h->tmB3, wg3, d->Cout, d->Cmid, swz, 64, sw, "W3");
+    if (rc == SLQ_OK) rc = encode_tiled_u8(&h->tmBd, wgd, (long long)h->n_tiles * 128, d->Cin, swz, 128, sw, "Wd");
     if (rc == SLQ_OK) {
       if (d->stride == 1) {
-        rc = bt_tiled_u8(&h->tmAd, x, h->M, d->Cin, swz, kTileM, sw, "x");
+        rc = encode_tiled_u8(&h->tmAd, x, h->M, d->Cin, swz, kTileM, sw, "x");
       } else {  // strided 1x1: the im2col-mode map walks every stride-th pixel
-        BtEncodeTiledFn enc;
-        BtEncodeIm2colFn enc2;
-        rc = bt_encoders(&enc, &enc2);
-        if (rc == SLQ_OK) {
-          cuuint64_t dims[4] = {(cuuint64_t)d->Cin, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->N};
-          cuuint64_t strides[3] = {(cuuint64_t)d->Cin, (cuuint64_t)d->W * d->Cin, (cuuint64_t)d->H * d->W * d->Cin};
-          int lower[2] = {0, 0}, upper[2] = {0, 0};
-          cuuint32_t es[4] = {1, (cuuint32_t)d->stride, (cuuint32_t)d->stride, 1};
-          const CUresult r = enc2(&h->tmAd, CU_TENSOR_MAP_DATA_TYPE_UINT8, 4, const_cast<uint8_t *>(x), dims, strides, lower, upper,
-                                  (cuuint32_t)swz, (cuuint32_t)kTileM, es, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-          if (r != CUDA_SUCCESS) {
-            set_error("cuTensorMapEncodeIm2col(x) failed: CUresult %d", (int)r);
-            rc = SLQ_ERR_CUDA;
-          }
-          int drv = 0;
-          if (rc == SLQ_OK && cudaDriverGetVersion(&drv) == cudaSuccess && drv <= 13010 &&
-              (long long)d->N * d->H * d->W * d->Cin < 131072)
-            reinterpret_cast<uint64_t *>(&h->tmAd)[1] &= ~(1ull << 21);  // same driver issue as conv_umma.cu
-        }
+        const int lower[2] = {0, 0}, upper[2] = {0, 0};
+        rc = encode_im2col_u8(&h->tmAd, x, d->N, d->H, d->W, d->Cin, lower, upper, d->stride, swz, kTileM, sw, "x");
       }
     }
     if (rc != SLQ_OK) {
@@ -613,7 +525,7 @@ extern "C" int slq_blocktail_launch(slq_blocktail *h, const slq_blocktail_epilog
   bt_plan(&d, h->swz, &stages, off);
   a.b3_off = off[0]; a.bd_off = off[1]; a.ring_off = off[2]; a.out_off = off[3]; a.prm_off = off[4]; a.bar_off = off[5];
   if (e->out_mode == SLQ_OUT_U8 && h->out_ptr != e->out) {
-    int rc = bt_tiled_u8(&h->tmO, e->out, h->M, d.Cout, 64, kTileM, CU_TENSOR_MAP_SWIZZLE_64B, "out");
+    int rc = encode_tiled_u8(&h->tmO, e->out, h->M, d.Cout, 64, kTileM, CU_TENSOR_MAP_SWIZZLE_64B, "out");
     if (rc != SLQ_OK) return rc;
     h->out_ptr = e->out;
   }

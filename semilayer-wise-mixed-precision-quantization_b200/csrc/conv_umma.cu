@@ -39,6 +39,7 @@
 #include <new>
 
 #include "conv_common.cuh"
+#include "tma_host.cuh"
 #include "umma_ptx.cuh"
 
 namespace slq {
@@ -182,13 +183,7 @@ struct KernelArgs {
 // fire-and-forget store (no atomics: their latency would distort the very thing being measured)
 constexpr int kTraceIssuers = 24;
 // trace_cap < 0 selects "wait statistics only": every role adds up the cycles it spends blocked in its
-// mbarrier waits and CTA 0 writes one total per role at the end (slot = role) -- no per-step overhead
-__device__ __forceinline__ void mbar_wait_stat(uint32_t bar, uint32_t parity, long long &sum, bool stats) {
-  if (!kDebugTrace || !stats) { mbar_wait(bar, parity); return; }
-  const long long t0 = clock64();  // try_wait itself may suspend the thread: time the whole wait
-  mbar_wait(bar, parity);
-  sum += clock64() - t0;
-}
+// mbarrier waits (mbar_wait_stat) and CTA 0 writes one total per role at the end (slot = role) -- no per-step overhead
 __device__ __forceinline__ void trace_ev(const KernelArgs &a, int issuer, int &n, int ev, int idx) {
   if (!kDebugTrace || a.trace == nullptr || a.trace_cap < 0 || blockIdx.x != 0) return;
   const int per = a.trace_cap / kTraceIssuers;
@@ -336,13 +331,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     mbar_init(stfree_bar(1), 1);
     fence_barrier_init();
   }
-  if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                     smem_u32((const void *)tmem_slot)),
-                 "r"(kTmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 2) tmem_alloc(tmem_slot, kTmemCols);
   // constant "ones" row group behind the B rows of every B tile:
   // row bn_cols = 0x01.., rows bn_cols+1 .. +15 = 0  (identical bytes are swizzle-invariant)
   if (ones_row) {
@@ -930,125 +919,35 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   }
   if (warp == 2) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
+    tmem_dealloc(tmem_base, kTmemCols);
   }
 }
 
 // ------------------------------------------------------------------------------------------
 // host side: tensor maps + launch
 // ------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *,
-                                  CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
-                                  CUtensorMapFloatOOBfill);
-typedef CUresult (*EncodeIm2colFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                   const cuuint64_t *, const int *, const int *, cuuint32_t, cuuint32_t,
-                                   const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static int get_encoders(EncodeTiledFn *tiled, EncodeIm2colFn *im2col) {
-  static EncodeTiledFn f_tiled = nullptr;
-  static EncodeIm2colFn f_im2col = nullptr;
-  if (!f_tiled || !f_im2col) {
-    void *p = nullptr;
-    cudaDriverEntryPointQueryResult qr;
-    SLQ_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qr));
-    if (qr != cudaDriverEntryPointSuccess || !p) {
-      set_error("cuTensorMapEncodeTiled not available from the driver");
-      return SLQ_ERR_CUDA;
-    }
-    f_tiled = (EncodeTiledFn)p;
-    p = nullptr;
-    SLQ_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeIm2col", &p, cudaEnableDefault, &qr));
-    if (qr != cudaDriverEntryPointSuccess || !p) {
-      set_error("cuTensorMapEncodeIm2col not available from the driver");
-      return SLQ_ERR_CUDA;
-    }
-    f_im2col = (EncodeIm2colFn)p;
-  }
-  *tiled = f_tiled;
-  *im2col = f_im2col;
-  return SLQ_OK;
-}
-
 // [M, Cout] u8 tensor (output or residual) as a tiled map with box = bn_ch channels x 128 pixels
 static int encode_out_map(CUtensorMap *tm, const void *ptr, const ConvGeom &g, const char *what) {
-  EncodeTiledFn enc_tiled;
-  EncodeIm2colFn enc_im2col;
-  int rc = get_encoders(&enc_tiled, &enc_im2col);
-  if (rc != SLQ_OK) return rc;
-  cuuint64_t dims[2] = {(cuuint64_t)g.Cout, (cuuint64_t)g.M};
-  cuuint64_t strides[1] = {(cuuint64_t)g.Cout};
-  cuuint32_t box[2] = {(cuuint32_t)g.bn_ch, (cuuint32_t)kTileM};
-  cuuint32_t es[2] = {1, 1};
-  CUresult r = enc_tiled(tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void *>(ptr), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE,
-                         g.bn_ch == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
-                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled(%s) failed: CUresult %d", what, (int)r);
-    return SLQ_ERR_CUDA;
-  }
-  return SLQ_OK;
+  return encode_tiled_u8(tm, ptr, g.M, g.Cout, g.bn_ch, kTileM,
+                         g.bn_ch == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, what);
 }
 
 static int build_tensor_maps(slq_conv *c) {
-  EncodeTiledFn enc_tiled;
-  EncodeIm2colFn enc_im2col;
-  int rc = get_encoders(&enc_tiled, &enc_im2col);
-  if (rc != SLQ_OK) return rc;
   const ConvGeom &g = c->g;
   const int swz = c->swizzle;
   const CUtensorMapSwizzle sw = swz == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
-  CUresult r;
   for (int wide = 0; wide <= (c->wide_ok ? 1 : 0); ++wide) {
     // B: GEMM-ready weights [gemm_rows, Ktot] u8, box = SWZ bytes of K x bn_cols rows (one map per tiling)
     const ConvGeom &gb = wide ? c->g_wide : c->g;
-    cuuint64_t dims[2] = {(cuuint64_t)gb.Ktot, (cuuint64_t)gb.gemm_rows};
-    cuuint64_t strides[1] = {(cuuint64_t)gb.Ktot};
-    cuuint32_t box[2] = {(cuuint32_t)swz, (cuuint32_t)gb.bn_cols};
-    cuuint32_t es[2] = {1, 1};
-    r = enc_tiled(wide ? &c->tmB_wide : &c->tmB, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, (void *)c->wg, dims, strides, box, es,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled(B) failed: CUresult %d", (int)r);
-      return SLQ_ERR_CUDA;
-    }
+    const int rc = encode_tiled_u8(wide ? &c->tmB_wide : &c->tmB, c->wg, gb.gemm_rows, gb.Ktot, swz, gb.bn_cols, sw, "B");
+    if (rc != SLQ_OK) return rc;
   }
-  if (!c->a_im2col) {  // A: [M, Cin] u8 (1x1 stride-1), box = SWZ channels x 128 pixels
-    cuuint64_t dims[2] = {(cuuint64_t)g.Cin, (cuuint64_t)g.M};
-    cuuint64_t strides[1] = {(cuuint64_t)g.Cin};
-    cuuint32_t box[2] = {(cuuint32_t)swz, (cuuint32_t)kTileM};
-    cuuint32_t es[2] = {1, 1};
-    r = enc_tiled(&c->tmA, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, (void *)c->in, dims, strides, box, es,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled(A) failed: CUresult %d", (int)r);
-      return SLQ_ERR_CUDA;
-    }
-  } else {  // A: NHWC u8 through im2col mode; base pixel = top-left tap of each output pixel
-    cuuint64_t dims[4] = {(cuuint64_t)g.Cin, (cuuint64_t)g.W, (cuuint64_t)g.H, (cuuint64_t)g.N};
-    cuuint64_t strides[3] = {(cuuint64_t)g.Cin, (cuuint64_t)g.W * g.Cin, (cuuint64_t)g.H * g.W * g.Cin};
-    int lower[2] = {-g.pad, -g.pad};                               // {W, H}
-    int upper[2] = {g.pad - (g.kw - 1), g.pad - (g.kh - 1)};       // {W, H}
-    cuuint32_t es[4] = {1, (cuuint32_t)g.stride, (cuuint32_t)g.stride, 1};
-    r = enc_im2col(&c->tmA, CU_TENSOR_MAP_DATA_TYPE_UINT8, 4, (void *)c->in, dims, strides, lower, upper,
-                   (cuuint32_t)swz, (cuuint32_t)kTileM, es, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeIm2col(A) failed: CUresult %d", (int)r);
-      return SLQ_ERR_CUDA;
-    }
-    // Known driver issue (<= 13.1): im2col maps of tensors below 128 KiB come back with bit 21 of
-    // the second descriptor word set and then fault; CUTLASS clears it the same way.
-    int drv = 0;
-    if (cudaDriverGetVersion(&drv) == cudaSuccess && drv <= 13010 &&
-        (long long)g.N * g.H * g.W * g.Cin < 131072)
-      reinterpret_cast<uint64_t *>(&c->tmA)[1] &= ~(1ull << 21);
-  }
-  return SLQ_OK;
+  if (!c->a_im2col)  // A: [M, Cin] u8 (1x1 stride-1), box = SWZ channels x 128 pixels
+    return encode_tiled_u8(&c->tmA, c->in, g.M, g.Cin, swz, kTileM, sw, "A");
+  // A: NHWC u8 through im2col mode; base pixel = top-left tap of each output pixel
+  const int lower[2] = {-g.pad, -g.pad};                          // {W, H}
+  const int upper[2] = {g.pad - (g.kw - 1), g.pad - (g.kh - 1)};  // {W, H}
+  return encode_im2col_u8(&c->tmA, c->in, g.N, g.H, g.W, g.Cin, lower, upper, g.stride, swz, kTileM, sw, "A");
 }
 
 static long long *g_trace = nullptr;  // slq_debug_set_trace
@@ -1057,13 +956,8 @@ void debug_trace_buffer(long long **buf, int *cap) { *buf = g_trace; *cap = g_tr
 
 template <int SWZ, bool W16, int OUT, int RES>
 static int launch_one(slq_conv *c, const EpiDev &e, int tma_out, cudaStream_t st) {
-  static bool attr_done[kMaxDevices] = {false};  // function attributes are per device
-  const int dev = current_device();
-  if (dev >= kMaxDevices || !attr_done[dev]) {
-    SLQ_CUDA(cudaFuncSetAttribute(conv_umma_kernel<SWZ, W16, OUT, RES>,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
-    if (dev < kMaxDevices) attr_done[dev] = true;
-  }
+  constexpr auto kernel = conv_umma_kernel<SWZ, W16, OUT, RES>;
+  SLQ_CUDA(set_smem_limit_once<kernel>(kSmemLimit));
   // K-heavy layers (weights streamed) without residual run 256-channel tiles
   const bool wide = c->wide_ok && e.res == nullptr && !W16;
   const ConvGeom &geom = wide ? c->g_wide : c->g;
@@ -1095,22 +989,7 @@ static int launch_one(slq_conv *c, const EpiDev &e, int tma_out, cudaStream_t st
   a.mma_warps_per_tile = (a.sp.mma_warps == 2 && a.num_grp >= 2 && !a.tile_alt) ? 2 : 1;
   a.m_tiles = ceil_div(geom.M, kTileM);
   a.tma_out = tma_out;
-  // Programmatic dependent launch: this grid's CTAs may start (barrier / TMEM set-up, resident weights)
-  // on an SM as soon as the previous kernel's CTA there has exited; griddepcontrol.wait in the kernel
-  // holds everything that touches activations until the previous grid has completed.
-  const bool pdl = true;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = (size_t)a.sp.total;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl ? 1 : 0;
-  SLQ_CUDA(cudaLaunchKernelEx(&cfg, conv_umma_kernel<SWZ, W16, OUT, RES>, c->tmA, wide ? c->tmB_wide : c->tmB, c->tmO,
-                              c->tmR, a));
+  SLQ_CUDA(launch_pdl(kernel, grid, kThreads, a.sp.total, st, c->tmA, wide ? c->tmB_wide : c->tmB, c->tmO, c->tmR, a));
   return SLQ_OK;
 }
 

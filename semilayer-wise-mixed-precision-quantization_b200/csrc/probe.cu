@@ -7,6 +7,7 @@
 // 8192).  bench.py times the launch with CUDA events -- once short (burst clocks) and once for >= 2 s
 // (sustained, under the power cap) -- and divides the conv kernels' achieved ops by it.
 #include "conv_common.cuh"
+#include "tma_host.cuh"
 #include "umma_ptx.cuh"
 
 namespace slq {
@@ -26,10 +27,7 @@ __global__ void __launch_bounds__(128, 1) probe_i8_kernel(int iters) {
     for (int i = 0; i < 8; ++i) mbar_init(smem_u32(&bars[i >> 2][i & 3]), 1);
     fence_barrier_init();
   }
-  if (w == 3) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(512) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (w == 3) tmem_alloc(&tmem_slot, 512);
   fence_proxy_async_smem();
   tc_fence_before();
   __syncthreads();
@@ -65,7 +63,7 @@ __global__ void __launch_bounds__(128, 1) probe_i8_kernel(int iters) {
   __syncthreads();
   if (w == 3) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512) : "memory");
+    tmem_dealloc(tmem, 512);
   }
 }
 
@@ -75,12 +73,7 @@ using namespace slq;
 
 extern "C" int slq_probe_i8_peak(int32_t iters, int64_t *ops_out, void *stream) {
   SLQ_CHECK_ARG(iters > 0 && (iters & 3) == 0, "slq_probe_i8_peak: iters must be a positive multiple of 4");
-  static bool attr_done[kMaxDevices] = {false};
-  const int dev = current_device();
-  if (dev < kMaxDevices && !attr_done[dev]) {
-    SLQ_CUDA(cudaFuncSetAttribute(probe_i8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kProbeSmem));
-    attr_done[dev] = true;
-  }
+  SLQ_CUDA(set_smem_limit_once<probe_i8_kernel>(kProbeSmem));
   const int ctas = sm_count();
   probe_i8_kernel<<<ctas, 128, kProbeSmem, (cudaStream_t)stream>>>(iters);
   SLQ_LAUNCH_CHECK();

@@ -28,6 +28,7 @@
 #include <new>
 
 #include "conv_common.cuh"
+#include "tma_host.cuh"
 #include "umma_ptx.cuh"
 
 struct slq_stem {
@@ -182,13 +183,7 @@ __global__ void __launch_bounds__(kSfThreads, 1) stem_fused_kernel(const StemArg
     }
     fence_barrier_init();
   }
-  if (warp == kSfBW + 8) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                     smem_u32((const void *)tmem_slot)),
-                 "r"(kSfTmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == kSfBW + 8) tmem_alloc(tmem_slot, kSfTmemCols);
   // zero the input ring (its pad columns are never written again) and stage weights + BN constants
   for (int i = threadIdx.x; i < kSfRingBytes / 16; i += blockDim.x)
     reinterpret_cast<uint4 *>(smem + kSfRingOff)[i] = make_uint4(0, 0, 0, 0);
@@ -419,7 +414,7 @@ __global__ void __launch_bounds__(kSfThreads, 1) stem_fused_kernel(const StemArg
   __syncthreads();
   if (warp == kSfBW + 8) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kSfTmemCols) : "memory");
+    tmem_dealloc(tmem_base, kSfTmemCols);
   }
 }
 
@@ -474,26 +469,6 @@ __global__ void stem_weights_ts_kernel(const float *__restrict__ w, float *__res
   wh[idx] = v;
 }
 
-__device__ __forceinline__ void bulk_copy_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void tmem_st4(uint32_t taddr, uint32_t r0, uint32_t r1, uint32_t r2, uint32_t r3) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};"
-               ::"r"(taddr), "r"(r0), "r"(r1), "r"(r2), "r"(r3) : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-// D[tmem] (+)= A[tmem] * B[smem], fp16 operands, fp32 accumulate
-__device__ __forceinline__ void umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc,
-                                            uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
 template <int IN>
 __global__ void __launch_bounds__(kTsThreads, 1) stem_ts_kernel(const __grid_constant__ CUtensorMap tmX, const StemArgs a) {
   extern __shared__ uint8_t smem_raw[];
@@ -531,11 +506,7 @@ __global__ void __launch_bounds__(kTsThreads, 1) stem_ts_kernel(const __grid_con
   }
   if (warp == 0) {
     if (lane == 0) prefetch_tmap(&tmX);
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                     smem_u32((const void *)tmem_slot)),
-                 "r"(kTsTmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(tmem_slot, kTsTmemCols);
   }
   // converted-row buffers: the pad columns are never written again; weights + BN constants
   for (int i = threadIdx.x; i < kTsRowBufBytes / 16; i += blockDim.x)
@@ -849,7 +820,7 @@ __global__ void __launch_bounds__(kTsThreads, 1) stem_ts_kernel(const __grid_con
   __syncthreads();
   if (warp == 0) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTsTmemCols) : "memory");
+    tmem_dealloc(tmem_base, kTsTmemCols);
   }
 }
 
@@ -890,26 +861,16 @@ extern "C" int slq_stem_create(int32_t N, int32_t H, int32_t W, void *workspace,
 #endif
   const int units_per_img = (s->Hp + kSfUnitRows - 1) / kSfUnitRows;
   s->num_ctas = (int)std::min<long long>((long long)N * units_per_img, sm_count());
-  static bool attr_done[kMaxDevices] = {false};
-  const int cur_dev = current_device();
-  if (cur_dev >= kMaxDevices || !attr_done[cur_dev]) {
-    cudaError_t e = cudaFuncSetAttribute(stem_fused_kernel<SLQ_IN_F32>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSfSmemBytes);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(stem_fused_kernel<SLQ_IN_F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSfSmemBytes);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(stem_fused_kernel<SLQ_IN_U8>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSfSmemBytes);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(stem_ts_kernel<SLQ_IN_F32>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTsSmemBytes);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(stem_ts_kernel<SLQ_IN_F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTsSmemBytes);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(stem_ts_kernel<SLQ_IN_U8>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTsSmemBytes);
-    if (e != cudaSuccess) {
-      delete s;
-      set_error("slq_stem_create: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-      return SLQ_ERR_CUDA;
-    }
-    if (cur_dev < kMaxDevices) attr_done[cur_dev] = true;
+  cudaError_t e = set_smem_limit_once<stem_fused_kernel<SLQ_IN_F32>>(kSfSmemBytes);
+  if (e == cudaSuccess) e = set_smem_limit_once<stem_fused_kernel<SLQ_IN_F16>>(kSfSmemBytes);
+  if (e == cudaSuccess) e = set_smem_limit_once<stem_fused_kernel<SLQ_IN_U8>>(kSfSmemBytes);
+  if (e == cudaSuccess) e = set_smem_limit_once<stem_ts_kernel<SLQ_IN_F32>>(kTsSmemBytes);
+  if (e == cudaSuccess) e = set_smem_limit_once<stem_ts_kernel<SLQ_IN_F16>>(kTsSmemBytes);
+  if (e == cudaSuccess) e = set_smem_limit_once<stem_ts_kernel<SLQ_IN_U8>>(kTsSmemBytes);
+  if (e != cudaSuccess) {
+    delete s;
+    set_error("slq_stem_create: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    return SLQ_ERR_CUDA;
   }
   *out = s;
   return SLQ_OK;
@@ -970,31 +931,15 @@ extern "C" int slq_stem_launch_in(slq_stem *s, const void *x, int32_t in_kind, c
   if (s->use_ts) {
     SLQ_CHECK_ARG(reinterpret_cast<uintptr_t>(x) % 16 == 0, "slq_stem_launch: the image must be 16-byte aligned");
     // the image as a 3-D tensor [3N planes][H][W]; one box = {W, 2 rows, 3 channels} = one input-row pair
-    typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                      const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                      CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    static EncodeTiledFn enc = nullptr;
-    if (!enc) {
-      void *fp = nullptr;
-      cudaDriverEntryPointQueryResult qr;
-      SLQ_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fp, cudaEnableDefault, &qr));
-      SLQ_CHECK_ARG(qr == cudaDriverEntryPointSuccess && fp, "cuTensorMapEncodeTiled not available from the driver");
-      enc = (EncodeTiledFn)fp;
-    }
     const int esz = in_kind == SLQ_IN_F32 ? 4 : (in_kind == SLQ_IN_F16 ? 2 : 1);
     CUtensorMap tmX;
-    cuuint64_t dims[3] = {(cuuint64_t)s->W, (cuuint64_t)s->H, (cuuint64_t)3 * s->N};
-    cuuint64_t strides[2] = {(cuuint64_t)s->W * esz, (cuuint64_t)s->H * s->W * esz};
-    cuuint32_t box[3] = {(cuuint32_t)s->W, 2, 3};
-    cuuint32_t es[3] = {1, 1, 1};
+    const cuuint64_t dims[3] = {(cuuint64_t)s->W, (cuuint64_t)s->H, (cuuint64_t)3 * s->N};
+    const cuuint64_t strides[2] = {(cuuint64_t)s->W * esz, (cuuint64_t)s->H * s->W * esz};
+    const cuuint32_t box[3] = {(cuuint32_t)s->W, 2, 3};
     const CUtensorMapDataType dt = in_kind == SLQ_IN_F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
                                    : (in_kind == SLQ_IN_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8);
-    const CUresult r = enc(&tmX, dt, 3, const_cast<void *>(x), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                           CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled(stem image) failed: CUresult %d", (int)r);
-      return SLQ_ERR_CUDA;
-    }
+    const int rc = encode_tiled(&tmX, dt, 3, x, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE, "stem image");
+    if (rc != SLQ_OK) return rc;
     if (in_kind == SLQ_IN_F32) stem_ts_kernel<SLQ_IN_F32><<<s->num_ctas, kTsThreads, kTsSmemBytes, st>>>(tmX, a);
     else if (in_kind == SLQ_IN_F16) stem_ts_kernel<SLQ_IN_F16><<<s->num_ctas, kTsThreads, kTsSmemBytes, st>>>(tmX, a);
     else stem_ts_kernel<SLQ_IN_U8><<<s->num_ctas, kTsThreads, kTsSmemBytes, st>>>(tmX, a);

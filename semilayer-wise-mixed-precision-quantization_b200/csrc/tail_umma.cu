@@ -18,6 +18,7 @@
 #include <algorithm>
 
 #include "conv_common.cuh"
+#include "tma_host.cuh"
 #include "umma_ptx.cuh"
 
 namespace slq {
@@ -105,16 +106,6 @@ constexpr int kFcTileBytes = 128 * 128;                     // 128 rows x 32 flo
 constexpr int kFcSmemBytes = 1024 + kFcStages * 2 * kFcTileBytes + 256;
 constexpr int kFcThreads = 192;                             // warp 0 TMA, warp 1 MMA, warps 2-5 epilogue
 
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                          uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
 __global__ void __launch_bounds__(kFcThreads, 1) fc_umma_kernel(const __grid_constant__ CUtensorMap tmAhi,
                                                                 const __grid_constant__ CUtensorMap tmAlo,
                                                                 const __grid_constant__ CUtensorMap tmBhi,
@@ -142,13 +133,7 @@ __global__ void __launch_bounds__(kFcThreads, 1) fc_umma_kernel(const __grid_con
     mbar_init(tfull_bar, 1);
     fence_barrier_init();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                     smem_u32((const void *)tmem_slot)),
-                 "r"(128)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, 128);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -217,7 +202,7 @@ __global__ void __launch_bounds__(kFcThreads, 1) fc_umma_kernel(const __grid_con
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(128) : "memory");
+    tmem_dealloc(tmem_base, 128);
   }
 }
 
@@ -231,35 +216,13 @@ __global__ void __launch_bounds__(256) fc_reduce_kernel(const float *__restrict_
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *,
-                                  CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
-                                  CUtensorMapFloatOOBfill);
-
+// [rows, K] fp32 matrix, box = 32 floats (128 bytes) x 128 rows
 static int encode_f32_rows(CUtensorMap *tm, const float *ptr, int rows, int K) {
-  static EncodeTiledFn enc = nullptr;
-  if (!enc) {
-    void *p = nullptr;
-    cudaDriverEntryPointQueryResult qr;
-    SLQ_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qr));
-    if (qr != cudaDriverEntryPointSuccess || !p) {
-      set_error("cuTensorMapEncodeTiled not available from the driver");
-      return SLQ_ERR_CUDA;
-    }
-    enc = (EncodeTiledFn)p;
-  }
-  cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)K * 4};
-  cuuint32_t box[2] = {32, 128};
-  cuuint32_t es[2] = {1, 1};
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float *>(ptr), dims, strides, box, es,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled(fc operand) failed: CUresult %d", (int)r);
-    return SLQ_ERR_CUDA;
-  }
-  return SLQ_OK;
+  const cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
+  const cuuint64_t strides[1] = {(cuuint64_t)K * 4};
+  const cuuint32_t box[2] = {32, 128};
+  return encode_tiled(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, ptr, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                      "fc operand");
 }
 
 static int fc_splits(int C) {
@@ -306,12 +269,7 @@ extern "C" int slq_tail_forward(const uint8_t *x, int32_t N, int32_t HW, int32_t
   if (rc == SLQ_OK) rc = encode_f32_rows(&tmBhi, fc_w, O, C);
   if (rc == SLQ_OK) rc = encode_f32_rows(&tmBlo, fc_w + (int64_t)O * C, O, C);
   if (rc != SLQ_OK) return rc;
-  static bool attr_done[kMaxDevices] = {false};
-  const int dev = current_device();
-  if (dev >= kMaxDevices || !attr_done[dev]) {
-    SLQ_CUDA(cudaFuncSetAttribute(fc_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFcSmemBytes));
-    if (dev < kMaxDevices) attr_done[dev] = true;
-  }
+  SLQ_CUDA(set_smem_limit_once<fc_umma_kernel>(kFcSmemBytes));
   const int splits = fc_splits(C);
   dim3 grid((unsigned)ceil_div(O, 128), (unsigned)ceil_div(N, 128), (unsigned)splits);
   fc_umma_kernel<<<grid, kFcThreads, kFcSmemBytes, st>>>(tmAhi, tmAlo, tmBhi, tmBlo, N, O, C / 32 / splits, partial);

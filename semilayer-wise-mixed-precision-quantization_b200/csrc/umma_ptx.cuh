@@ -1,5 +1,5 @@
 // csrc/umma_ptx.cuh -- thin inline-PTX wrappers for the Blackwell (sm_100a) async machinery used by
-// the tcgen05 kernels: mbarrier, TMA (tiled + im2col), tcgen05.mma / commit / ld, TMEM fences,
+// the tcgen05 kernels: mbarrier, TMA (tiled + im2col), tcgen05.mma / commit / ld / st, TMEM allocation and fences,
 // and the K-major shared-memory matrix descriptor.
 #pragma once
 #include <cuda.h>
@@ -53,6 +53,14 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
       __trap();
     }
   }
+}
+// mbar_wait that, when `stats` is on (debug build only), adds the cycles spent blocked to `sum`: the wait
+// statistics of slq_debug_set_trace
+__device__ __forceinline__ void mbar_wait_stat(uint32_t bar, uint32_t parity, long long &sum, bool stats) {
+  if (!kDebugTrace || !stats) { mbar_wait(bar, parity); return; }
+  const long long t0 = clock64();  // try_wait itself may suspend the thread: time the whole wait
+  mbar_wait(bar, parity);
+  sum += clock64() - t0;
 }
 // programmatic dependent launch: blocks until the grids this one depends on have completed and flushed
 __device__ __forceinline__ void grid_dependency_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
@@ -143,6 +151,37 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t desc_a, uint6
       ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate), "r"(0), "r"(0), "r"(0), "r"(0)
       : "memory");
 }
+// D[tmem] (+)= A[tmem] * B[smem], fp16 operands, fp32 accumulate
+__device__ __forceinline__ void umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc,
+                                            uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// D[tmem] (+)= A[smem] * B[smem], tf32 operands, fp32 accumulate, single CTA
+__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                          uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// one whole warp: allocates ncols TMEM columns, writes their base address to *slot (shared memory) and gives up
+// the CTA's right to allocate more
+__device__ __forceinline__ void tmem_alloc(const volatile uint32_t *slot, uint32_t ncols) {
+  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void *)slot)),
+               "r"(ncols) : "memory");
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+// one whole warp, the one that allocated
+__device__ __forceinline__ void tmem_dealloc(uint32_t tmem_base, uint32_t ncols) {
+  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(ncols) : "memory");
+}
 __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap *map, uint32_t bar, int c0,
                                             int c1, int c2) {
   asm volatile(
@@ -187,6 +226,11 @@ __device__ __forceinline__ uint32_t tmem_ld1(uint32_t taddr) {
 __device__ __forceinline__ void tmem_ld_wait() {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
+__device__ __forceinline__ void tmem_st4(uint32_t taddr, uint32_t r0, uint32_t r1, uint32_t r2, uint32_t r3) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};"
+               ::"r"(taddr), "r"(r0), "r"(r1), "r"(r2), "r"(r3) : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // K-major shared-memory matrix descriptor for a tile whose rows are SWZ bytes long and stored with
 // the SWZ-byte TMA/UMMA swizzle (8-row groups of 8*SWZ bytes, tile base aligned to 1024 B).
