@@ -346,7 +346,8 @@ SLQ_API int slq_tail_forward(const uint8_t *x, int32_t N, int32_t HW, int32_t C,
  * `tmp` is one device uint32 of scratch, zeroed by the call.                                     */
 SLQ_API int slq_absmax_scale(const float *y, int64_t n, float *act_scales, int32_t id, int32_t qmax,
                      uint32_t *tmp, void *stream);
-/* out[i] = clamp(rint(y[i] / act_scales[id]), 0, 255)  (is_signed: clamp to [-127, 127], s8) */
+/* out[i] = clamp(rint(y[i] / act_scales[id]), 0, 255)  (is_signed: clamp to [-128, 127], s8: the range of
+ * every s8 producer, cvt.rni.sat.s8, and of slq_oracle.requant_s8) */
 SLQ_API int slq_quantize_act(const float *y, int64_t n, const float *act_scales, int32_t id,
                      int32_t is_signed, uint8_t *out, void *stream);
 
