@@ -346,6 +346,29 @@ SLQ_API int slq_tail_forward(const uint8_t *x, int32_t N, int32_t HW, int32_t C,
  * `tmp` is one device uint32 of scratch, zeroed by the call.                                     */
 SLQ_API int slq_absmax_scale(const float *y, int64_t n, float *act_scales, int32_t id, int32_t qmax,
                      uint32_t *tmp, void *stream);
+
+/* Histogram calibration (opt-in; abs-max above is the default).  A scale set by the single largest element
+ * only grows with more data; a threshold read from the distribution of |y| does not.
+ * slq_act_histogram ADDS the counts of |y[0..n)| (y 4-byte aligned, any offset) to histogram `id` of
+ * hist [.][bins + 1] (device uint64, zeroed by the caller before the first call):
+ *   hist[id][0]      exact zeros (either sign)
+ *   hist[id][1 + j]  0 < |y| with j = min(trunc(fp32(|y| * fp32(bins / range[id]))), bins - 1): values at or
+ *                    above range[id] land in the last bin
+ * slq_hist_scales turns histograms [n_tensors][bins + 1] into act_scales[0..n_tensors), one CTA per tensor, in
+ * fp64.  Candidate thresholds T_k = fp32(fp32(range * k) / bins), k = 1..bins (T_bins == range).
+ *   SLQ_CALIB_PERCENTILE  smallest k with zeros + n_0 + .. + n_{k-1} >= ceil(percentile / 100 * total),
+ *                         total including the zeros; 0 < percentile <= 100
+ *   SLQ_CALIB_MSE         k minimising sum_j n_j * (c_j - Q(c_j))^2 over the bin centres c_j = (j + 0.5) * range / bins,
+ *                         Q(v) = D * min(rint(v / D), qmax), D = T_k / qmax; exact ties go to the larger k
+ *   act_scales[t] = fp32(fp32(T_k / qmax[t]) * headroom), or 1.0 when the tensor has no non-zero element.
+ * bins: a power of two, at most 2048.  Counts are integers: both results are deterministic.             */
+#define SLQ_CALIB_PERCENTILE 1
+#define SLQ_CALIB_MSE 2
+SLQ_API int slq_act_histogram(const float *y, int64_t n, const float *range, int32_t id, int32_t bins,
+                              uint64_t *hist, void *stream);
+SLQ_API int slq_hist_scales(const uint64_t *hist, int32_t n_tensors, int32_t bins, const float *range,
+                            const int32_t *qmax, int32_t method, double percentile, float headroom,
+                            float *act_scales, void *stream);
 /* out[i] = clamp(rint(y[i] / act_scales[id]), 0, 255)  (is_signed: clamp to [-128, 127], s8: the range of
  * every s8 producer, cvt.rni.sat.s8, and of slq_oracle.requant_s8) */
 SLQ_API int slq_quantize_act(const float *y, int64_t n, const float *act_scales, int32_t id,

@@ -187,32 +187,66 @@ class ResNet(nn.Module):
         activation quantisation, or re-calibration noise lands on top of the effect being measured."""
         self._slq_donor = other
 
-    def slq_calibrate(self, batches, headroom=1.0):
+    CALIB_METHODS = ("absmax", "percentile", "mse")
+    CALIB_BINS = 2048
+
+    def slq_calibrate(self, batches, headroom=1.0, method="absmax", percentile=99.99):
         """Explicit calibration of the static per-tensor activation scales (the reference never quantises
-        activations, SURVEY.md F2, so this call has no counterpart there): running abs-max over ``batches``
-        (a tensor, a list of tensors, or a loader of (x, y) pairs; CUDA or host), times ``headroom``.
+        activations, SURVEY.md F2, so this call has no counterpart there) over ``batches`` (a tensor, a list of
+        tensors, or a loader of (x, y) pairs; CUDA or host), times ``headroom``:
+          * ``"absmax"``      running abs-max over the batches (the default);
+          * ``"percentile"``  the ``percentile``-th percentile of |y| over the batches, zeros included;
+          * ``"mse"``         the clipping threshold with the least squared quantisation error of |y|.
+        The last two read a 2048-bin histogram of every layer output, whose range comes from an abs-max pass
+        over the same batches: they iterate ``batches`` twice, so a one-shot iterator is refused.
         The scales then stay fixed -- through weight changes, state_dict reloads and later batches -- until
         the next slq_calibrate().  Without this call the first forward calibrates on its own batch."""
-        import slq_engine
+        import slq_lib as L
+        if method not in self.CALIB_METHODS:
+            raise ValueError("slq_calibrate: method %r is not one of %s" % (method, ", ".join(self.CALIB_METHODS)))
         if torch.is_tensor(batches):
             batches = [batches]
+        hist = method != "absmax"
+        if hist and iter(batches) is batches:
+            raise TypeError("slq_calibrate(method=%r) reads the batches twice: pass a list or a re-iterable "
+                            "loader, not a one-shot iterator" % method)
+        first, eng = True, None
+        for eng, x, n in self._calib_batches(batches):
+            # histogram methods: the abs-max pass only sets each tensor's range, over the images actually given
+            eng.calibrate(x, accumulate=not first, headroom=1.0 if hist else headroom, images=n if hist else None)
+            first = False
+        if first:
+            raise ValueError("slq_calibrate: no batches")
+        if not hist:
+            return
+        bins = self.CALIB_BINS
+        qmax = eng.act_qmax().to(torch.float32)
+        rng = eng.act_scales * qmax
+        counts = torch.zeros((len(eng.act), bins + 1), dtype=torch.int64, device=eng.device)
+        for e, x, n in self._calib_batches(batches):
+            if e is not eng:
+                raise ValueError("slq_calibrate: the batches changed shape between the two passes")
+            eng.histogram(x, counts, rng, bins, images=n)
+        eng.hist_scales(counts, rng, bins, L.CALIB_PERCENTILE if method == "percentile" else L.CALIB_MSE,
+                        percentile, headroom)
+
+    def _calib_batches(self, batches):
+        """(engine, batch on the device padded to the engine's batch size, images in it) per calibration batch."""
+        import slq_engine
         dev = self.conv1.weight.device
-        first = True
         for item in batches:
             x = item[0] if isinstance(item, (tuple, list)) else item
             x = x.to(dev, non_blocking=True)
-            cap = slq_engine.engine_batch(self, x.shape[0])
-            if x.shape[0] < cap:
+            n = x.shape[0]
+            cap = slq_engine.engine_batch(self, n)
+            if n < cap:
                 xp = x.new_zeros((cap,) + tuple(x.shape[1:]))
-                xp[:x.shape[0]] = x
+                xp[:n] = x
                 x = xp
             eng = self.slq_engine(x)
             eng.sync_weights(force=self._slq_dirty)
             self._slq_dirty = False
-            eng.calibrate(x, accumulate=not first, headroom=headroom)
-            first = False
-        if first:
-            raise ValueError("slq_calibrate: no batches")
+            yield eng, x, n
 
     def forward(self, x):
         if not x.is_cuda:

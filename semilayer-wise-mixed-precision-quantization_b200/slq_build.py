@@ -14,7 +14,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libslq_b200.so")
 STAMP = os.path.join(HERE, "build", "sources.sha256")
 SOURCES = ["quantizer.cu", "layers.cu", "conv_umma.cu", "stem_umma.cu", "eval_tail.cu", "probe.cu", "tail_umma.cu",
-           "block_tail.cu", "tma_host.cu"]
+           "block_tail.cu", "tma_host.cu", "calib.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden",

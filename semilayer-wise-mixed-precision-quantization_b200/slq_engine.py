@@ -549,32 +549,66 @@ class Engine:
         self.in_kind = kind
         return x.contiguous()
 
-    def calibrate(self, x, accumulate=False, headroom=1.0):
+    def calibrate(self, x, accumulate=False, headroom=1.0, images=None):
         """One pass with fp32 layer outputs: every activation tensor's static scale becomes
         absmax/255 (u8) or absmax/127 (s8) of this batch, times ``headroom``; with ``accumulate`` the
         larger of that and the scale it already has (running abs-max over several batches).  Each layer is
         then launched again in its quantised output mode, so the pass leaves exactly the bytes in HBM that
-        forward(x) produces (and every later layer is calibrated on what it will really see)."""
+        forward(x) produces (and every later layer is calibrated on what it will really see).
+        ``images``: only the first that many samples of x count (a padded short batch); None = all N."""
+        lib = self.lib
+        accumulate = accumulate and self.calibrated
+        sc, tmp = self.act_scales.data_ptr(), self.absmax_tmp.data_ptr()
+        old = self.act_scales.clone() if accumulate else None
+
+        def observe(st, y, n, idx, qmax):
+            L.check(lib.slq_absmax_scale(y, n, sc, idx, qmax, tmp, st))
+            if headroom != 1.0:
+                self.act_scales[idx:idx + 1].mul_(headroom)
+            if old is not None:
+                torch.maximum(self.act_scales[idx:idx + 1], old[idx:idx + 1], out=self.act_scales[idx:idx + 1])
+
+        self._calib_walk(x, observe, images)
+        self.calibrated = True
+
+    def act_qmax(self):
+        """Largest code of every activation tensor (device int32): 127 for s8 tensors, 255 for u8 ones."""
+        return torch.tensor([127 if s else 255 for s in self.act_signed], dtype=torch.int32, device=self.device)
+
+    def histogram(self, x, hist, rng, bins, images=None):
+        """The calibration pass of ``calibrate`` with the scales in force left as they are: adds |y| of every
+        layer output to its histogram (slq_act_histogram; hist [tensors, bins + 1] uint64, rng [tensors] fp32)."""
+        lib = self.lib
+
+        def observe(st, y, n, idx, qmax):
+            L.check(lib.slq_act_histogram(y, n, rng.data_ptr(), idx, bins, hist.data_ptr(), st))
+
+        self._calib_walk(x, observe, images)
+
+    def hist_scales(self, hist, rng, bins, method, percentile=99.99, headroom=1.0):
+        """Every activation scale from its histogram, in place (slq_hist_scales): captured graphs stay valid."""
+        with torch.cuda.device(self.device):
+            L.check(self.lib.slq_hist_scales(hist.data_ptr(), len(self.act), bins, rng.data_ptr(),
+                                             self.act_qmax().data_ptr(), method, percentile, headroom,
+                                             self.act_scales.data_ptr(), L.current_stream(self.device)))
+        self.calibrated = True
+
+    def _calib_walk(self, x, observe, images=None):
+        """stem -> schedule: each layer once with fp32 output into f32_scratch, observe(stream, ptr, n, id, qmax)
+        on it, then again in its quantised mode.  n covers the first ``images`` samples (NHWC: a prefix)."""
         lib = self.lib
         x = self._check_x(x)
         if any(op.handle is None for op in self.ops):
             raise RuntimeError("engine has no packed weights yet (call sync_weights())")
-        accumulate = accumulate and self.calibrated
+        images = self.N if images is None else images
+        if not 0 < images <= self.N:
+            raise ValueError("images=%d outside 1..%d" % (images, self.N))
         with torch.cuda.device(self.device), torch.no_grad():
             st = L.current_stream(self.device)
-            sc, tmp, f32 = self.act_scales.data_ptr(), self.absmax_tmp.data_ptr(), self.f32_scratch
-            old = self.act_scales.clone() if accumulate else None
-
-            def settle(idx):  # scale idx was just written by slq_absmax_scale
-                if headroom != 1.0:
-                    self.act_scales[idx:idx + 1].mul_(headroom)
-                if old is not None:
-                    torch.maximum(self.act_scales[idx:idx + 1], old[idx:idx + 1], out=self.act_scales[idx:idx + 1])
-
-            n0 = self.act[0].numel()
-            self._stem(x.data_ptr(), f32.data_ptr(), L.OUT_F32, st)
-            L.check(lib.slq_absmax_scale(f32.data_ptr(), n0, sc, 0, 255, tmp, st))
-            settle(0)
+            f32 = self.f32_scratch.data_ptr()
+            n0 = self.act[0].numel() // self.N * images
+            self._stem(x.data_ptr(), f32, L.OUT_F32, st)
+            observe(st, f32, n0, 0, 255)
             self._stem(x.data_ptr(), self.act[0].data_ptr(), L.OUT_U8, st)
             for item in self.schedule:
                 op = item[1].op3 if item[0] == "tail" else item[1]   # the layer whose output tensor this writes
@@ -582,15 +616,11 @@ class Engine:
                     # the identity tensor does not exist on this path; its scale is still kept current for the day
                     # the block falls back to two launches (conv3 restored to fp32 weights)
                     dop = item[1].dop
-                    self.launch_item(("conv", dop), st, L.OUT_F32, f32.data_ptr())
-                    L.check(lib.slq_absmax_scale(f32.data_ptr(), dop.M * dop.Cout, sc, dop.out_id, 127, tmp, st))
-                    settle(dop.out_id)
-                self.launch_item(item, st, L.OUT_F32, f32.data_ptr())
-                L.check(lib.slq_absmax_scale(f32.data_ptr(), op.M * op.Cout, sc, op.out_id,
-                                             127 if op.signed else 255, tmp, st))
-                settle(op.out_id)
+                    self.launch_item(("conv", dop), st, L.OUT_F32, f32)
+                    observe(st, f32, dop.M * dop.Cout // self.N * images, dop.out_id, 127)
+                self.launch_item(item, st, L.OUT_F32, f32)
+                observe(st, f32, op.M * op.Cout // self.N * images, op.out_id, 127 if op.signed else 255)
                 self.launch_item(item, st)
-        self.calibrated = True
 
     def forward(self, x):
         """Static-scale inference pass: stem -> conv launches -> tail.  Returns the engine's
