@@ -71,7 +71,11 @@ def codes_ohwi(meta, cout, cin, k):
 class ConvCase:
     """One conv layer on the device, built through the C ABI exactly like slq_engine does."""
 
-    def __init__(self, N, H, cin, cout, k, stride, bits, seed=0, impl=None, a_mode=0, device="cuda", packed_b=False):
+    def __init__(self, N, H, cin, cout, k, stride, bits, seed=0, impl=None, a_mode=0, device="cuda", packed_b=False,
+                 x=None):
+        """bits: per output channel, any of 2/4/6/8 (quantised rows) or 32 (an fp32 row: 16-bit codes, two limbs).
+        x: the input as a u8 NHWC [N, H, H, cin] device tensor (made on the device; self.x, the host copy the
+        numpy oracle reads, is then None); None draws it from `seed` on the host."""
         import slq_engine
         import slq_lib as L
         self.L = L
@@ -81,11 +85,15 @@ class ConvCase:
         self.pad = k // 2
         self.w, self.meta = make_weights(cout, cin, k, bits, seed)
         self.w16 = 1 if max(m[0] for m in self.meta) > 8 else 0
-        rng = np.random.default_rng(seed + 1)
-        self.x = rng.integers(0, 256, (N, H, H, cin), dtype=np.uint8)
-        self.xd = torch.from_numpy(self.x).to(device)
+        if x is None:
+            rng = np.random.default_rng(seed + 1)
+            self.x = rng.integers(0, 256, (N, H, H, cin), dtype=np.uint8)
+            self.xd = torch.from_numpy(self.x).to(device)
+        else:
+            assert x.dtype == torch.uint8 and tuple(x.shape) == (N, H, H, cin) and x.is_contiguous()
+            self.x, self.xd = None, x
         # per-pixel channel sums of the input (what the producing layer's epilogue accumulates)
-        self.rowsum = torch.from_numpy(self.x.astype(np.int64).sum(-1).astype(np.int32).reshape(-1)).to(device)
+        self.rowsum = self.xd.sum(-1, dtype=torch.int32).reshape(-1)
         wd = torch.from_numpy(self.w.reshape(cout, -1)).to(device)
         (bit, z, s, bits_host, _exact), = slq_engine.classify_weights([wd])
         self.bits_dev, self.z_dev, self.s_dev, self.bits_host = bit, z, s, bits_host
@@ -126,37 +134,59 @@ class ConvCase:
         return acc, None, S
 
     # ---- device side ----
-    def run_acc(self):
+    def _in_rowsum(self, in_rowsum, in_planes):
+        """The launch's rowsum fields: in_rowsum is a [planes, plane_stride] int32 device tensor whose first
+        in_planes planes (default: all) sum to the input's per-pixel channel sums; None = the one exact plane."""
+        rs = self.rowsum.view(1, -1) if in_rowsum is None else in_rowsum
+        assert rs.dim() == 2 and rs.dtype == torch.int32 and rs.is_contiguous()
+        return rs, rs.shape[0] if in_planes is None else in_planes, rs.shape[1]
+
+    def launch_acc(self, in_rowsum=None, in_planes=None):
+        """SLQ_OUT_ACC launch; returns the device tensors (out [M, Cout or 2*Cout] int32, S [M] int32) unsynchronised."""
         L = self.L
+        rs, planes, stride = self._in_rowsum(in_rowsum, in_planes)
         ncol = self.cout * (2 if self.w16 else 1)
         out = torch.full((self.M, ncol), -7, dtype=torch.int32, device=self.device)
         S = torch.full((self.M,), -7, dtype=torch.int32, device=self.device)
         e = L.Epilogue(None, None, None, None, 0, 0, -1, None, 0, out.data_ptr(), S.data_ptr(), L.OUT_ACC, 0,
-                       self.rowsum.data_ptr(), None, 1, self.rowsum.numel())
+                       rs.data_ptr(), None, planes, stride)
         L.check(L.lib().slq_conv_launch(self.handle, ctypes.byref(e), L.current_stream()))
+        return out, S
+
+    def run_acc(self):
+        out, S = self.launch_acc()
         torch.cuda.synchronize()
         return out.cpu().numpy(), S.cpu().numpy()
 
-    def run_epi(self, mode, wscale, zf, bias, scales, in_id, out_id, res=None, res_id=-1, res_signed=0, relu=1):
+    def launch_epi(self, mode, wscale, zf, bias, scales, in_id, out_id, res=None, res_id=-1, res_signed=0, relu=1,
+                   in_rowsum=None, in_planes=None, out=None):
+        """One epilogue launch; the vectors and res may be numpy arrays or device tensors.  out: the output
+        buffer (default: a fresh one filled with a sentinel).  Returns the device output unsynchronised and
+        sets self.out_rowsum (U8 launches: [slq_conv_rowsum_planes, M], filled with -3 before the launch)."""
         L = self.L
         dev = self.device
-        t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+        t = lambda a: a if torch.is_tensor(a) else torch.from_numpy(np.ascontiguousarray(a)).to(dev)
         ws, zz, bb, sc = t(wscale), t(zf), t(bias), t(scales)
         rs = t(res) if res is not None else None
-        if mode == L.OUT_F32:
+        if out is None and mode == L.OUT_F32:
             out = torch.full((self.M, self.cout), float("nan"), dtype=torch.float32, device=dev)
-        else:
+        elif out is None:
             out = torch.full((self.M, self.cout), 77, dtype=torch.uint8, device=dev)
         planes = L.lib().slq_conv_rowsum_planes(self.handle, 1 if res is not None else 0)
         self.out_rowsum = (torch.full((max(planes, 1), self.M), -3, dtype=torch.int32, device=dev)
                            if mode == L.OUT_U8 else None)
+        irs, in_planes, in_stride = self._in_rowsum(in_rowsum, in_planes)
         e = L.Epilogue(ws.data_ptr(), zz.data_ptr(), bb.data_ptr(), sc.data_ptr(), in_id, out_id, res_id,
-                       L.ptr(rs), res_signed, out.data_ptr(), None, mode, relu, self.rowsum.data_ptr(),
-                       L.ptr(self.out_rowsum), 1, self.rowsum.numel())
+                       L.ptr(rs), res_signed, out.data_ptr(), None, mode, relu, irs.data_ptr(),
+                       L.ptr(self.out_rowsum), in_planes, in_stride)
         L.check(L.lib().slq_conv_launch(self.handle, ctypes.byref(e), L.current_stream()))
+        return out
+
+    def run_epi(self, mode, wscale, zf, bias, scales, in_id, out_id, res=None, res_id=-1, res_signed=0, relu=1):
+        out = self.launch_epi(mode, wscale, zf, bias, scales, in_id, out_id, res, res_id, res_signed, relu)
         torch.cuda.synchronize()
         got = out.cpu().numpy()
-        if self.out_rowsum is not None and self.desc.impl == L.IMPL_UMMA:
+        if self.out_rowsum is not None and self.desc.impl == self.L.IMPL_UMMA:
             # the side tensor the next layer's epilogue gathers its window sums from
             # (one plane per n-tile of the launch; their sum is the channel sum of the pixel)
             want = got.astype(np.int64).sum(1)
