@@ -360,10 +360,25 @@ SLQ_API int slq_absmax_scale(const float *y, int64_t n, float *act_scales, int32
  *                         total including the zeros; 0 < percentile <= 100
  *   SLQ_CALIB_MSE         k minimising sum_j n_j * (c_j - Q(c_j))^2 over the bin centres c_j = (j + 0.5) * range / bins,
  *                         Q(v) = D * min(rint(v / D), qmax), D = T_k / qmax; exact ties go to the larger k
+ *   SLQ_CALIB_ENTROPY     k minimising the KL divergence D_k (TensorRT's and pytorch-quantization's entropy
+ *                         calibrator; bins >= 128).  n_j = hist[1 + j], N = sum_j n_j (zeros left out: they
+ *                         quantise to 0 at every threshold), nq = qmax + 1 levels; candidates k = 128..bins:
+ *                           o_k = sum_{j >= k} n_j (outliers), clipped onto the last bin:
+ *                             P_j = n_j (j < k - 1), P_{k-1} = n_{k-1} + o_k
+ *                           group(j) = floor(j * nq / k) (integers); m_g = sum of n_j over group g, c_g = its
+ *                             bins with n_j > 0; Q_j = m_g / c_g where n_j > 0, else 0 (sum Q = N - o_k)
+ *                           D_k = sum_{P_j > 0} (P_j / N) ln((P_j / N) / (Q_j / (N - o_k))); +inf when some
+ *                             P_j > 0 has Q_j = 0 (n_{k-1} = 0 < o_k, or N == o_k); D_bins is finite
+ *                         exact ties go to the larger k.  The device sums, per candidate, in fp64 and in
+ *                         increasing j over the bins with n_j > 0:
+ *                           D_k = (sum_j P_j * ln((P_j * (c_g * (N - o_k))) / (m_g * N))) / N,  g = group(j)
+ *                         so a bin with P_j == Q_j adds exactly 0 when o_k == 0.
  *   act_scales[t] = fp32(fp32(T_k / qmax[t]) * headroom), or 1.0 when the tensor has no non-zero element.
- * bins: a power of two, at most 2048.  Counts are integers: both results are deterministic.             */
+ * bins: a power of two, at most 2048.  Counts are integers (below 2^53) and every fp64 sum runs in a fixed
+ * order: the results are deterministic.                                                                 */
 #define SLQ_CALIB_PERCENTILE 1
 #define SLQ_CALIB_MSE 2
+#define SLQ_CALIB_ENTROPY 3
 SLQ_API int slq_act_histogram(const float *y, int64_t n, const float *range, int32_t id, int32_t bins,
                               uint64_t *hist, void *stream);
 SLQ_API int slq_hist_scales(const uint64_t *hist, int32_t n_tensors, int32_t bins, const float *range,

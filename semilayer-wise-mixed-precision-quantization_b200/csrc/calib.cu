@@ -1,8 +1,12 @@
 // csrc/calib.cu -- histogram calibration of the static activation scales (include/slq.h section 3):
 //   * act_histogram_kernel: |y| of one fp32 layer output into a uint64 histogram (HBM-bound)
 //   * hist_scales_kernel:   one CTA per tensor, histogram -> percentile or MSE threshold -> scale (fp64)
+//   * hist_entropy_kernel:  one CTA per tensor, histogram -> entropy (KL-divergence) threshold -> scale (fp64)
 // The binning rule is exact fp32 and the counts are integers, so the result is deterministic and
-// tests/calib_oracle.py (act_histogram, hist_scale) restates it bit for bit.
+// tests/calib_oracle.py (act_histogram, hist_scale) restates it bit for bit; tests/calib_entropy_oracle.py restates
+// the entropy rule.
+#include <math_constants.h>
+
 #include <algorithm>
 
 #include "common.cuh"
@@ -84,6 +88,28 @@ __device__ __forceinline__ float hist_threshold(float range, int k, int bins) {
 
 constexpr int kScaleThreads = 256;
 
+// Arg-min of (err, k) over the CTA, exact ties to the larger k; k == 0 marks a thread without a candidate.  Every
+// thread of the CTA calls this once and gets the winning k.
+__device__ int cta_argmin_larger_k(double best, int kb) {
+  __shared__ double sh_best_err[kScaleThreads / 32];
+  __shared__ int sh_best_k[kScaleThreads / 32];
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    const double oe = __shfl_xor_sync(0xffffffffu, best, off);
+    const int ok = __shfl_xor_sync(0xffffffffu, kb, off);
+    if (ok != 0 && (kb == 0 || oe < best || (oe == best && ok > kb))) best = oe, kb = ok;
+  }
+  if ((threadIdx.x & 31) == 0) sh_best_err[threadIdx.x >> 5] = best, sh_best_k[threadIdx.x >> 5] = kb;
+  __syncthreads();
+  best = sh_best_err[0], kb = sh_best_k[0];
+  for (int w = 1; w < kScaleThreads / 32; ++w) {
+    const double oe = sh_best_err[w];
+    const int ok = sh_best_k[w];
+    if (ok != 0 && (kb == 0 || oe < best || (oe == best && ok > kb))) best = oe, kb = ok;
+  }
+  return kb;
+}
+
 __global__ void __launch_bounds__(kScaleThreads) hist_scales_kernel(const unsigned long long *__restrict__ hist,
                                                                    int bins, const float *__restrict__ range,
                                                                    const int32_t *__restrict__ qmax_arr, int method,
@@ -92,8 +118,6 @@ __global__ void __launch_bounds__(kScaleThreads) hist_scales_kernel(const unsign
   // the non-empty bins of this tensor, compacted: bin centre and count (zeros contribute no error)
   __shared__ double sh_c[kHistMaxBins], sh_n[kHistMaxBins];
   __shared__ int sh_nnz;
-  __shared__ double sh_best_err[kScaleThreads / 32];
-  __shared__ int sh_best_k[kScaleThreads / 32];
   const int t = blockIdx.x;
   const unsigned long long *h = hist + (long long)t * (bins + 1);
   const float rng = range[t];
@@ -143,25 +167,75 @@ __global__ void __launch_bounds__(kScaleThreads) hist_scales_kernel(const unsign
       }
       if (kb == 0 || err <= best) best = err, kb = k;  // k rises along the loop: ties go to the larger k
     }
-    // arg-min over the CTA; exact ties -> larger k
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) {
-      const double oe = __shfl_xor_sync(0xffffffffu, best, off);
-      const int ok = __shfl_xor_sync(0xffffffffu, kb, off);
-      if (ok != 0 && (kb == 0 || oe < best || (oe == best && ok > kb))) best = oe, kb = ok;
-    }
-    if ((threadIdx.x & 31) == 0) sh_best_err[threadIdx.x >> 5] = best, sh_best_k[threadIdx.x >> 5] = kb;
-    __syncthreads();
+    k_best = cta_argmin_larger_k(best, kb);
     if (threadIdx.x != 0) return;
-    best = sh_best_err[0], kb = sh_best_k[0];
-    for (int w = 1; w < kScaleThreads / 32; ++w) {
-      const double oe = sh_best_err[w];
-      const int ok = sh_best_k[w];
-      if (ok != 0 && (kb == 0 || oe < best || (oe == best && ok > kb))) best = oe, kb = ok;
-    }
-    k_best = kb;
   }
   act_scales[t] = __fmul_rn(__fdiv_rn(hist_threshold(rng, k_best, bins), (float)qmax), headroom);
+}
+
+constexpr int kEntropyStartBin = 128;  // first candidate k of the entropy rule (pytorch-quantization's start_bin)
+
+// The entropy (KL-divergence) rule of include/slq.h section 3, one CTA per tensor: every candidate k on its own
+// thread, O(k) fp64 work from the prefix sums of the counts, then the CTA arg-min.
+__global__ void __launch_bounds__(kScaleThreads) hist_entropy_kernel(const unsigned long long *__restrict__ hist,
+                                                                    int bins, const float *__restrict__ range,
+                                                                    const int32_t *__restrict__ qmax_arr,
+                                                                    float headroom, float *__restrict__ act_scales) {
+  // n_j, and M[j] = n_0 + .. + n_{j-1}, C[j] = bins with n > 0 among 0 .. j-1: a group's m_g and c_g in O(1)
+  // (counts below 2^53: exact in fp64)
+  __shared__ double sh_n[kHistMaxBins], sh_m[kHistMaxBins + 1];
+  __shared__ int sh_c[kHistMaxBins + 1];
+  const int t = blockIdx.x;
+  const unsigned long long *h = hist + (long long)t * (bins + 1);
+  for (int j = threadIdx.x; j < bins; j += blockDim.x) sh_n[j] = (double)h[1 + j];
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double m = 0.0;
+    int c = 0;
+    for (int j = 0; j < bins; ++j) {
+      sh_m[j] = m, sh_c[j] = c;
+      m += sh_n[j], c += sh_n[j] != 0.0;
+    }
+    sh_m[bins] = m, sh_c[bins] = c;
+  }
+  __syncthreads();
+  const double N = sh_m[bins];
+  if (N == 0.0) {
+    if (threadIdx.x == 0) act_scales[t] = 1.0f;
+    return;
+  }
+  const int qmax = qmax_arr[t];
+  // nq >= k splits every candidate into single bins, so capping nq at bins changes no group and keeps g * k
+  // within int
+  const int nq = min(qmax, bins - 1) + 1;
+  double best = 0.0;
+  int kb = 0;
+  for (int k = kEntropyStartBin + threadIdx.x; k <= bins; k += blockDim.x) {
+    const double kept = sh_m[k], o = N - kept;  // o_k: the outliers clipped onto bin k - 1
+    double d = CUDART_INF;
+    if (o == 0.0 || sh_n[k - 1] != 0.0) {
+      double acc = 0.0;
+      for (int g = 0, lo = 0; g < nq; ++g) {
+        const int hi = ((g + 1) * k + nq - 1) / nq;  // group g: bins ceil(g k / nq) .. ceil((g + 1) k / nq) - 1
+        const double m = sh_m[hi] - sh_m[lo];
+        if (m != 0.0) {
+          const double num = __dmul_rn((double)(sh_c[hi] - sh_c[lo]), kept), den = __dmul_rn(m, N);
+          for (int j = lo; j < hi; ++j) {
+            const double n = sh_n[j];
+            if (n == 0.0) continue;
+            const double p = j == k - 1 ? n + o : n;
+            acc = __dadd_rn(acc, __dmul_rn(p, log(__ddiv_rn(__dmul_rn(p, num), den))));
+          }
+        }
+        lo = hi;
+      }
+      d = __ddiv_rn(acc, N);
+    }
+    if (kb == 0 || d <= best) best = d, kb = k;  // k rises along the loop: ties go to the larger k
+  }
+  const int k_best = cta_argmin_larger_k(best, kb);
+  if (threadIdx.x == 0)
+    act_scales[t] = __fmul_rn(__fdiv_rn(hist_threshold(range[t], k_best, bins), (float)qmax), headroom);
 }
 
 }  // namespace slq
@@ -189,12 +263,20 @@ extern "C" int slq_hist_scales(const uint64_t *hist, int32_t n_tensors, int32_t 
                                float *act_scales, void *stream) {
   SLQ_CHECK_ARG(hist && range && qmax && act_scales && n_tensors > 0, "slq_hist_scales: bad argument");
   SLQ_CHECK_ARG(hist_bins_ok(bins), "slq_hist_scales: bins=%d must be a power of two in [1, %d]", bins, kHistMaxBins);
-  SLQ_CHECK_ARG(method == SLQ_CALIB_PERCENTILE || method == SLQ_CALIB_MSE, "slq_hist_scales: method %d", method);
+  SLQ_CHECK_ARG(method == SLQ_CALIB_PERCENTILE || method == SLQ_CALIB_MSE || method == SLQ_CALIB_ENTROPY,
+                "slq_hist_scales: method %d", method);
+  SLQ_CHECK_ARG(method != SLQ_CALIB_ENTROPY || bins >= kEntropyStartBin,
+                "slq_hist_scales: entropy needs at least %d bins, got bins=%d", kEntropyStartBin, bins);
   SLQ_CHECK_ARG(method != SLQ_CALIB_PERCENTILE || (percentile > 0.0 && percentile <= 100.0),
                 "slq_hist_scales: percentile %g outside (0, 100]", percentile);
   SLQ_CHECK_ARG(headroom > 0.f, "slq_hist_scales: headroom must be positive");
-  hist_scales_kernel<<<n_tensors, kScaleThreads, 0, (cudaStream_t)stream>>>(
-      reinterpret_cast<const unsigned long long *>(hist), bins, range, qmax, method, percentile, headroom, act_scales);
+  const auto *h = reinterpret_cast<const unsigned long long *>(hist);
+  if (method == SLQ_CALIB_ENTROPY)
+    hist_entropy_kernel<<<n_tensors, kScaleThreads, 0, (cudaStream_t)stream>>>(h, bins, range, qmax, headroom,
+                                                                              act_scales);
+  else
+    hist_scales_kernel<<<n_tensors, kScaleThreads, 0, (cudaStream_t)stream>>>(h, bins, range, qmax, method,
+                                                                             percentile, headroom, act_scales);
   SLQ_LAUNCH_CHECK();
   return SLQ_OK;
 }

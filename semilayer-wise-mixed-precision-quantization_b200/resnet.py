@@ -187,7 +187,7 @@ class ResNet(nn.Module):
         activation quantisation, or re-calibration noise lands on top of the effect being measured."""
         self._slq_donor = other
 
-    CALIB_METHODS = ("absmax", "percentile", "mse")
+    CALIB_METHODS = ("absmax", "percentile", "mse", "entropy")
     CALIB_BINS = 2048
 
     def slq_calibrate(self, batches, headroom=1.0, method="absmax", percentile=99.99):
@@ -196,8 +196,11 @@ class ResNet(nn.Module):
         tensors, or a loader of (x, y) pairs; CUDA or host), times ``headroom``:
           * ``"absmax"``      running abs-max over the batches (the default);
           * ``"percentile"``  the ``percentile``-th percentile of |y| over the batches, zeros included;
-          * ``"mse"``         the clipping threshold with the least squared quantisation error of |y|.
-        The last two read a 2048-bin histogram of every layer output, whose range comes from an abs-max pass
+          * ``"mse"``         the clipping threshold with the least squared quantisation error of |y|;
+          * ``"entropy"``     the clipping threshold whose quantised distribution of |y| has the least KL
+                              divergence from the observed one (TensorRT's and pytorch-quantization's entropy
+                              calibrator; zeros left out, candidates from bin 128 of 2048 up).
+        The last three read a 2048-bin histogram of every layer output, whose range comes from an abs-max pass
         over the same batches: they iterate ``batches`` twice, so a one-shot iterator is refused.
         The scales then stay fixed -- through weight changes, state_dict reloads and later batches -- until
         the next slq_calibrate().  Without this call the first forward calibrates on its own batch."""
@@ -206,7 +209,9 @@ class ResNet(nn.Module):
             raise ValueError("slq_calibrate: method %r is not one of %s" % (method, ", ".join(self.CALIB_METHODS)))
         if torch.is_tensor(batches):
             batches = [batches]
-        hist = method != "absmax"
+        # threshold rule of slq_hist_scales per histogram method; None: abs-max, no histogram
+        rule = {"percentile": L.CALIB_PERCENTILE, "mse": L.CALIB_MSE, "entropy": L.CALIB_ENTROPY}.get(method)
+        hist = rule is not None
         if hist and iter(batches) is batches:
             raise TypeError("slq_calibrate(method=%r) reads the batches twice: pass a list or a re-iterable "
                             "loader, not a one-shot iterator" % method)
@@ -227,8 +232,7 @@ class ResNet(nn.Module):
             if e is not eng:
                 raise ValueError("slq_calibrate: the batches changed shape between the two passes")
             eng.histogram(x, counts, rng, bins, images=n)
-        eng.hist_scales(counts, rng, bins, L.CALIB_PERCENTILE if method == "percentile" else L.CALIB_MSE,
-                        percentile, headroom)
+        eng.hist_scales(counts, rng, bins, rule, percentile, headroom)
 
     def _calib_batches(self, batches):
         """(engine, batch on the device padded to the engine's batch size, images in it) per calibration batch."""

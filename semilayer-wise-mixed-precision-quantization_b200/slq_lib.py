@@ -17,7 +17,7 @@ IMPL_UMMA, IMPL_SIMT = 0, 1
 A_AUTO, A_IM2COL, A_TILED = 0, 1, 2
 OUT_U8, OUT_F32, OUT_ACC, OUT_S8 = 0, 1, 2, 3
 IN_F32, IN_F16, IN_U8 = 0, 1, 2  # element type of the image handed to the stem (slq_stem_launch_in)
-CALIB_PERCENTILE, CALIB_MSE = 1, 2  # threshold rule of slq_hist_scales
+CALIB_PERCENTILE, CALIB_MSE, CALIB_ENTROPY = 1, 2, 3  # threshold rule of slq_hist_scales
 
 _i32, _i64, _vp = ctypes.c_int32, ctypes.c_int64, ctypes.c_void_p
 

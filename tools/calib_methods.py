@@ -1,11 +1,13 @@
 """tools/calib_methods.py -- what each activation-scale calibration method (``net.slq_calibrate(method=...)``) buys:
 
   * held-out logits parity (rel-L2 against the reference's fp32 fake-quant forward, top-1 agreement) of "absmax",
-    "percentile" and "mse" on BASELINE.json's R50 @256 and R34 @128 configurations, calibrated on 1 batch and on
-    8 batches (the held-out batches are those of tests/test_baseline_configs_gpu.py);
+    "percentile", "mse" and "entropy" on BASELINE.json's R50 @256 and R34 @128 configurations, calibrated on
+    1 batch and on 8 batches (the held-out batches are those of tests/test_baseline_configs_gpu.py);
   * calibration wall time of each method (batches already on the device; host clock around a synchronised call);
   * slq_act_histogram throughput on the largest fp32 layer output of R50 @256 ([256, 56, 56, 256], 822 MB: larger
-    than L2), next to a device-to-device copy of the same tensor timed in the same run.
+    than L2), next to a device-to-device copy of the same tensor timed in the same run;
+  * slq_hist_scales time per threshold rule (CUDA events) on the real histograms of every activation tensor of
+    R50 @256, taken from one calibration walk.
 
 The card's name and power limit are read in the same run and written beside the numbers.
 usage: python tools/calib_methods.py --out profiles/calib_methods.json
@@ -28,7 +30,7 @@ import slq_lib as L  # noqa: E402
 import slq_oracle as so  # noqa: E402
 from helpers import build_p0_model, rel_l2  # noqa: E402
 
-METHODS = ("absmax", "percentile", "mse")
+METHODS = ("absmax", "percentile", "mse", "entropy")
 CONFIGS = [("resnet50", 256, 11, (12, 13)), ("resnet34", 128, 21, (22, 23))]
 
 
@@ -112,12 +114,47 @@ def hist_bandwidth(iters=20):
     return res
 
 
+def hist_scales_time(iters=20):
+    lib = L.lib()
+    net = build_p0_model("resnet50", "cuda")
+    x = batch(256, 11).cuda()
+    net.slq_calibrate(x)  # abs-max: the ranges of the histogram pass
+    eng = next(iter(net._slq_engines.values()))
+    q = eng.act_qmax()
+    rng = eng.act_scales * q.to(torch.float32)
+    bins = net.CALIB_BINS
+    hist = torch.zeros((len(eng.act), bins + 1), dtype=torch.int64, device="cuda")
+    eng.histogram(x, hist, rng, bins)
+    out = torch.empty(len(eng.act), dtype=torch.float32, device="cuda")
+    st = L.current_stream()
+    rules = {"percentile": L.CALIB_PERCENTILE, "mse": L.CALIB_MSE, "entropy": L.CALIB_ENTROPY}
+
+    def launch(rule):
+        L.check(lib.slq_hist_scales(hist.data_ptr(), len(eng.act), bins, rng.data_ptr(), q.data_ptr(), rule, 99.99,
+                                    1.0, out.data_ptr(), st))
+
+    res = {"tensors": len(eng.act), "bins": bins, "iters": iters}
+    for rep in range(2):  # the rules alternated, twice
+        for name, rule in rules.items():
+            for _ in range(3):
+                launch(rule)
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            for _ in range(iters):
+                launch(rule)
+            e1.record()
+            torch.cuda.synchronize()
+            res.setdefault(name + "_us", []).append(e0.elapsed_time(e1) / iters * 1e3)
+    print(json.dumps(res), flush=True)
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", required=True)
     args = ap.parse_args()
     torch.cuda.set_device(0)
-    out = {"card": card(), "histogram": hist_bandwidth(), "parity": []}
+    out = {"card": card(), "histogram": hist_bandwidth(), "hist_scales": hist_scales_time(), "parity": []}
     for arch, n, cs, held in CONFIGS:
         for n_calib in (1, 8):
             out["parity"] += parity(arch, n, cs, held, n_calib)
