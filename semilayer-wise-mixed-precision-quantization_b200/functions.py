@@ -272,96 +272,231 @@ def _to_device(net, device):
 _RESIDENT = {"key": None, "loader": None, "batches": None}
 
 
-def _resident_batches(data_loader, device):
+def _resident_batches(data_loader, device, rank=0, world=1):
     """An IN-MEMORY loader (a list / tuple of (x, y) host tensors, e.g. imagenet.synthetic_loader or a calibration
     set) is copied to the device once and the copies are reused by the following evaluations, as long as the
     loader object and its tensors are unchanged (pointer + version counter per tensor).  Every candidate of a
     sweep evaluates the same batches: the pageable 38.5 MB per 64 images were copied again for each of them.
-    Streaming loaders (anything else) are passed through."""
+    With ``world`` > 1 only the batches ``rank`` owns (batch i belongs to rank i % world) are returned, and only
+    those are copied.  Streaming loaders (anything else) are passed through."""
+    if not isinstance(data_loader, (list, tuple)):
+        return data_loader
+    mine = data_loader if world == 1 else data_loader[rank::world]
     dev = torch.device(device)
-    if dev.type != "cuda" or not isinstance(data_loader, (list, tuple)) or os.environ.get("SLQ_NO_RESIDENT_LOADER"):
-        return data_loader  # (a writer that goes through ``x.data`` bumps no version counter: set the variable then)
+    if dev.type != "cuda" or os.environ.get("SLQ_NO_RESIDENT_LOADER"):
+        return mine  # (a writer that goes through ``x.data`` bumps no version counter: set the variable then)
     try:
-        sig = tuple((x.data_ptr(), x._version, tuple(x.shape), y.data_ptr(), y._version) for x, y in data_loader)
+        sig = tuple((x.data_ptr(), x._version, tuple(x.shape), y.data_ptr(), y._version) for x, y in mine)
     except Exception:
-        return data_loader
-    if any(x.is_cuda for x, _y in data_loader):
-        return data_loader
-    key = (id(data_loader), str(dev), sig)
+        return mine
+    if any(x.is_cuda for x, _y in mine):
+        return mine
+    key = (id(data_loader), str(dev), rank, world, sig)
     if _RESIDENT["key"] != key:
-        _RESIDENT["batches"] = [(x.to(device), y.to(device)) for x, y in data_loader]
+        _RESIDENT["batches"] = [(x.to(device), y.to(device)) for x, y in mine]
         _RESIDENT["key"], _RESIDENT["loader"] = key, data_loader  # the reference keeps id() from being recycled
     return _RESIDENT["batches"]
 
 
-def _evaluate(net, device, data_loader, ref_outputs=None, want_probs=True):
+_RANK_LOADER = {"key": None, "loader": None, "batches": None}
+
+
+def _subset_loader(data_loader, batch_ids):
+    """A DataLoader over ``data_loader``'s dataset that yields exactly its batches ``batch_ids`` (the loader reads the
+    dataset in order: batch i is the indices [i*B, (i+1)*B)), with the same collate function, workers and pinning."""
+    from torch.utils.data import DataLoader
+    B, N = data_loader.batch_size, len(data_loader.dataset)
+    kw = dict(num_workers=data_loader.num_workers, collate_fn=data_loader.collate_fn,
+              pin_memory=data_loader.pin_memory, worker_init_fn=data_loader.worker_init_fn,
+              multiprocessing_context=data_loader.multiprocessing_context, timeout=data_loader.timeout)
+    if data_loader.num_workers > 0:
+        kw.update(prefetch_factor=data_loader.prefetch_factor, persistent_workers=data_loader.persistent_workers)
+    return DataLoader(data_loader.dataset, batch_sampler=[list(range(i * B, min((i + 1) * B, N))) for i in batch_ids],
+                      **kw)
+
+
+def _rank_loader(data_loader, rank, world):
+    """For a torch DataLoader that reads its dataset in order (a SequentialSampler, as ``shuffle=False`` makes): a
+    DataLoader that yields only the batches of ``rank`` -- the same tensors the full loader yields for them, read and
+    decoded by this rank's workers alone.  Cached per (loader, rank) like the resident batches.  None for any other
+    loader."""
+    from torch.utils.data import DataLoader, SequentialSampler
+    if not (isinstance(data_loader, DataLoader) and isinstance(data_loader.sampler, SequentialSampler)
+            and data_loader.sampler.data_source is data_loader.dataset and data_loader.batch_size is not None):
+        return None
+    key = (id(data_loader), rank, world, len(data_loader.dataset))
+    if _RANK_LOADER["key"] != key:
+        _RANK_LOADER["batches"] = _subset_loader(data_loader, range(rank, len(data_loader), world))
+        _RANK_LOADER["key"], _RANK_LOADER["loader"] = key, data_loader
+    return _RANK_LOADER["batches"]
+
+
+def _rank_batches(data_loader, device, rank, world):
+    """The batches ``rank`` of ``world`` evaluates, batch i belonging to rank i % world: -> (number of batches, or None
+    when only a full pass tells; iterable of (i, (x, y)); first, a callable returning batch 0 when the iterable leaves
+    it out, else None; batch 0's (H, W), or None when unknown without reading it).  Only a loader that is neither in
+    memory nor a DataLoader reading its dataset in order is iterated in full; the caller skips other ranks' batches."""
+    if world > 1 and isinstance(data_loader, (list, tuple)):
+        n = len(data_loader)
+        return n, zip(range(rank, n, world), _resident_batches(data_loader, device, rank, world)), \
+            lambda: data_loader[0], tuple(data_loader[0][0].shape[2:]) if n else None
+    sub = _rank_loader(data_loader, rank, world) if world > 1 else None
+    if sub is not None:
+        n = len(data_loader)
+        return n, zip(range(rank, n, world), sub), lambda: next(iter(_subset_loader(data_loader, [0]))), None
+    return None, enumerate(_resident_batches(data_loader, device)), None, None
+
+
+def _calibrate_on_batch0(net, device, batch0, hw):
+    """What a single process's first forward does to the activation scales: when the net holds none for batch 0's
+    image size (``hw``; None: any size), calibrate them on batch 0."""
+    if not net.slq_calibrated(hw):
+        with torch.no_grad():
+            net(batch0()[0].to(device))
+
+
+def _all_gather(t, dist, world):
+    """all_gather of one equally shaped tensor per rank -> the world tensors, in rank order: NCCL on the current CUDA
+    device, any other backend through the host."""
+    dev = torch.device("cuda", torch.cuda.current_device()) if dist.get_backend() == "nccl" else torch.device("cpu")
+    t = t.to(dev)
+    bufs = [torch.empty_like(t) for _ in range(world)]
+    dist.all_gather(bufs, t)
+    return bufs
+
+
+_PROB_DTYPES = (torch.float32, torch.float64, torch.float16, torch.bfloat16)
+_FUSED, _HOST = 1, 2  # which route a rank's batches took (bit mask, gathered with the records)
+
+
+def _evaluate(net, device, data_loader, ref_outputs=None, want_probs=True, shard=True):
     """One pass over the loader: -> (acc, loss, [softmax per batch], KL(ref_outputs || outputs) or None).
 
     On CUDA the whole tail of every batch -- argmax, cross-entropy, softmax and, when ``ref_outputs`` (the
     stored softmax outputs of the un-quantised model) is given, the per-sample KL divergence -- is ONE fused
-    kernel pass (slq_eval_tail) that accumulates into four doubles on the device; they are read back ONCE
-    at the end (the reference synchronises three times per evaluation, functions.py:129, and KLdiv loops
-    over every sample in Python, functions.py:142-146).  CPU tensors take the stock-torch route."""
+    kernel pass (slq_eval_tail) that writes the batch's record of four doubles on the device; the records are read
+    back ONCE at the end and folded in batch order on the host, which adds the same values in the same order as one
+    running accumulator would (the reference synchronises three times per evaluation, functions.py:129, and KLdiv
+    loops over every sample in Python, functions.py:142-146).  CPU tensors take the stock-torch route, whose
+    per-batch values are folded with the reference's fp32 adds.
+
+    With ``shard`` and torch.distributed initialised with a world size above 1, the evaluation is data-parallel by
+    batch: batch i is run (forward and tail) by rank i % world only, one all_gather exchanges the records and, when
+    ``want_probs``, a second one the probabilities, and every rank returns what a single process returns, bit for
+    bit.  Every rank must therefore make the same evaluations in the same order, as for make_semilayers."""
     _to_device(net, device)
     net.eval()
-    lib = None
-    accum = None
-    data_loader = _resident_batches(data_loader, device)
-    labels, preds, outputs = [], [], []
-    loss_sum, count, n_img = 0, 0, 0
-    kl_sum, kl_n = None, 0
+    dist, rank, world = _dist() if shard else (None, 0, 1)
+    n, batches, first, hw0 = _rank_batches(data_loader, device, rank, world)
+    try:
+        slots = max(1, -(-len(data_loader) // world))
+    except TypeError:
+        slots = 64
+    lib, dev_recs, host_recs, outputs = None, None, [], []
     criterion = torch.nn.CrossEntropyLoss()
-    for bi, (x, y) in enumerate(data_loader):
+    # An uncalibrated engine calibrates its activation scales on its first batch, which in one process is batch 0.
+    # Every other rank, one that owns no batch too, runs batch 0 through the net first: then all ranks hold the same
+    # scales, in this evaluation and in any unsharded one that follows (the sweep's candidates).
+    calib0 = world > 1 and rank != 0 and torch.device(device).type == "cuda" and hasattr(net, "slq_calibrated")
+    if calib0 and first is not None and n:
+        _calibrate_on_batch0(net, device, first, hw0)
+    n_seen = 0
+    for bi, (x, y) in batches:
+        n_seen = bi + 1
+        if bi % world != rank:
+            if bi == 0 and calib0:
+                _calibrate_on_batch0(net, device, lambda: (x, y), tuple(x.shape[2:]))
+            continue
         x, y = x.to(device), y.to(device)
         with torch.no_grad():
             out = net(x)
         ref = ref_outputs[bi] if ref_outputs is not None else None
         if _fused_tail_ok(out) and (ref is None or (_fused_tail_ok(ref) and ref.shape == out.shape)):
-            if accum is None:
+            k = len(outputs)
+            if dev_recs is None or k == dev_recs.shape[0]:
+                more = torch.zeros((slots, 4), dtype=torch.float64, device=out.device)
+                dev_recs = more if dev_recs is None else torch.cat([dev_recs, more])
                 lib = L.lib()
-                accum = torch.zeros(4, dtype=torch.float64, device=out.device)
             B, C = out.shape
             y64 = y.to(torch.int64).contiguous()
             probs = torch.empty_like(out) if want_probs else None
             rows = torch.empty(3 * B, dtype=torch.float32, device=out.device)
             with torch.cuda.device(out.device):
                 L.check(lib.slq_eval_tail(out.data_ptr(), y64.data_ptr(), B, C, L.ptr(probs), L.ptr(ref),
-                                          rows.data_ptr(), accum.data_ptr(), L.current_stream(out.device)))
-            outputs.append(probs)
-            n_img += B
-        else:  # stock torch ops, exactly the reference's sequence
+                                          rows.data_ptr(), dev_recs[k].data_ptr(), L.current_stream(out.device)))
+        else:  # stock torch ops, the reference's per-batch values: (#correct, batch-mean CE, sum of KL, images)
             with torch.no_grad():
-                preds.append(out.max(1)[1])
-                loss_sum = loss_sum + criterion(out, y)
-                p = torch.softmax(out, dim=1)
-                outputs.append(p)
-                if ref is not None:
-                    kl = (ref * (ref / p).log()).sum(dim=1)
-                    kl_sum = kl.sum() if kl_sum is None else kl_sum + kl.sum()
-                    kl_n += kl.numel()
-            labels.append(y)
-        count += 1
-    if accum is not None:
-        if labels:
-            raise RuntimeError("evaluate: the loader mixed CUDA and host batches")
-        a = accum.cpu().numpy()  # the one device->host read of the evaluation
-        acc = float(np.float32(a[0]) / np.float32(n_img))
-        loss = float(np.float32(a[1]) / np.float32(count))
-        kl = float(np.float32(a[2] / a[3])) if ref_outputs is not None else None
+                probs = torch.softmax(out, dim=1)
+                kl = (ref * (ref / probs).log()).sum(dim=1).sum() if ref is not None else out.new_zeros(())
+                host_recs.append(torch.stack([(out.max(1)[1] == y).sum().double(), criterion(out, y).double(),
+                                              kl.double(), out.new_tensor(float(y.numel()), dtype=torch.float64)]))
+        outputs.append(probs)
+    n = n_seen if n is None else n
+    route = (_FUSED if dev_recs is not None else 0) | (_HOST if host_recs else 0)
+    recs = dev_recs[:len(outputs)] if route == _FUSED else torch.stack(host_recs) if route == _HOST else None
+    if world == 1:
+        if recs is None or route == _FUSED | _HOST:
+            _evaluation_error(route)
+        a = recs.cpu().numpy()  # the one device->host read of the evaluation
+    else:
+        m = -(-n // world)  # batches per rank, the last ones padded
+        C = outputs[0].shape[1] if outputs and want_probs else 0
+        dtype = _PROB_DTYPES.index(outputs[0].dtype) if outputs and want_probs else 0
+        send = torch.zeros((m + 1, 4), dtype=torch.float64, device=torch.device(device))
+        if recs is not None:
+            send[:len(outputs)] = recs.to(send.device)
+        send[m] = torch.tensor([route, C, dtype, 0], dtype=torch.float64)
+        gathered = torch.stack(_all_gather(send, dist, world)).cpu().numpy()  # the one device->host read
+        route = int(np.bitwise_or.reduce(gathered[:, m, 0].astype(np.int64)))
+        if route not in (_FUSED, _HOST):
+            _evaluation_error(route)
+        a = gathered[:, :m].transpose(1, 0, 2).reshape(-1, 4)[:n]  # row i = batch i (rank i % world, slot i // world)
+        if want_probs:
+            C, dtype = int(gathered[:, m, 1].max()), _PROB_DTYPES[int(gathered[:, m, 2].max())]
+            sizes = a[:, 3].astype(np.int64)
+            probs = torch.zeros((m, int(sizes.max()), C), dtype=dtype, device=torch.device(device))
+            for k, p in enumerate(outputs):
+                probs[k, :p.shape[0]] = p
+            bufs = [b.to(probs.device) for b in _all_gather(probs, dist, world)]
+            outputs = [bufs[i % world][i // world, :sizes[i]] for i in range(n)]
+        else:
+            outputs = [None] * n
+    if route == _FUSED:
+        s = [0.0, 0.0, 0.0, 0.0]  # the running accumulator of one process, fed the same records in the same order
+        for rec in a.tolist():
+            for j in range(4):
+                s[j] += rec[j]
+        acc = float(np.float32(s[0]) / np.float32(s[3]))
+        loss = float(np.float32(s[1]) / np.float32(n))
+        kl = float(np.float32(s[2] / s[3])) if ref_outputs is not None else None
         return acc, loss, outputs, kl
-    labels, preds = torch.cat(labels), torch.cat(preds)
-    acc = (labels == preds).float().sum() / len(labels)
-    kl = (kl_sum / kl_n).item() if kl_sum is not None else None
-    return acc.item(), (loss_sum / count).item(), outputs, kl
+    f32 = lambda v: torch.tensor(v, dtype=torch.float32)  # noqa: E731 -- the host records are fp32 values
+    loss_sum, kl_sum = 0, None
+    for rec in a.tolist():
+        loss_sum = loss_sum + f32(rec[1])
+        kl_sum = f32(rec[2]) if kl_sum is None else kl_sum + f32(rec[2])
+    images = int(a[:, 3].sum())
+    acc = f32(float(a[:, 0].sum())) / images  # an exact count, as the reference's sum of 0/1 floats
+    kl = (kl_sum / images).item() if ref_outputs is not None else None
+    return acc.item(), (loss_sum / n).item(), outputs, kl
+
+
+def _evaluation_error(route):
+    if route == _FUSED | _HOST:
+        raise RuntimeError("evaluate: the loader mixed CUDA and host batches")
+    raise RuntimeError("evaluate: the loader yielded no batches")
 
 
 def evaluate_loss(net, device, data_loader):
-    """Mean-of-batch-means cross-entropy (reference functions.py:45-82; unused by the mains)."""
+    """Mean-of-batch-means cross-entropy (reference functions.py:45-82; unused by the mains).  Data-parallel over
+    the ranks of a torch.distributed job like evaluate_acc_loss_softmax."""
     return _evaluate(net, device, data_loader, want_probs=False)[1]
 
 
 def evaluate_acc_loss_softmax(net, device, data_loader):
-    """-> (accuracy, mean-of-batch-means CE loss, [softmax per batch])  (reference functions.py:84-129)."""
+    """-> (accuracy, mean-of-batch-means CE loss, [softmax per batch])  (reference functions.py:84-129).
+    Under torch.distributed (world size > 1) each rank runs only the batches i with i % world == rank and every
+    rank returns the full result, identical to a single process's; every rank must make the same calls."""
     acc, loss, outputs, _kl = _evaluate(net, device, data_loader)
     return acc, loss, outputs
 
@@ -445,10 +580,7 @@ def _semilayer_runs(listminus, listplus):
 
 def _gather_values(values, flags, dist, world):
     """ONE all_gather of [values | error flags]; entry i comes from its owner rank i % world."""
-    both = torch.cat([values, flags])
-    dev = torch.device("cuda", torch.cuda.current_device()) if dist.get_backend() == "nccl" else torch.device("cpu")
-    bufs = [torch.zeros_like(both, device=dev) for _ in range(world)]
-    dist.all_gather(bufs, both.to(dev))
+    bufs = _all_gather(torch.cat([values, flags]), dist, world)
     n = values.numel()
     for index in range(n):
         src = bufs[index % world].cpu()
@@ -487,7 +619,7 @@ def make_semilayers(arch, net, device, originaloutputs, listminus, listplus, met
     # delta-loss needs the un-quantised loss from logits (the stored softmax underflows to exact zeros on
     # random-init R34/R50, which is what makes KL NaN there): one more evaluation of the caller's net,
     # before candidate 0 mutates it
-    base = _evaluate(net, device, imagenet.val_loader, want_probs=False)[1] if metric == "dloss" else None
+    base = _evaluate(net, device, imagenet.val_loader, want_probs=False, shard=False)[1] if metric == "dloss" else None
     values = torch.zeros(len(semilayers), dtype=torch.float64)
     flags = torch.zeros(len(semilayers), dtype=torch.float64)
     work, first_error = None, None
@@ -534,7 +666,7 @@ def make_semilayers(arch, net, device, originaloutputs, listminus, listplus, met
                 want_kl = metric == "kl"
                 _acc, loss, _after, kl = _evaluate(cand, device, imagenet.val_loader,
                                                    ref_outputs=originaloutputs if want_kl else None,
-                                                   want_probs=False)
+                                                   want_probs=False, shard=False)
                 val = (loss - base) if metric == "dloss" else kl / param
                 values[index] = val
                 print(rows[0][4], 'bit', 'semilayer-No.', index, 'layernumber=', rows[0][2], 'channels=', len(rows),
@@ -658,7 +790,7 @@ def make_deltaloss_table(arch, net, device, data_loader, bits=(8, 6, 4), layers=
     dist, rank, world = _dist() if shard else (None, 0, 1)
     net.to(device)
     net.eval()
-    base = _evaluate(net, device, data_loader, want_probs=False)[1]
+    base = _evaluate(net, device, data_loader, want_probs=False, shard=False)[1]
     cols = []
     for lnum, conv in quantized_convs(arch, net):
         if layers is not None and lnum not in layers:
@@ -676,7 +808,8 @@ def make_deltaloss_table(arch, net, device, data_loader, bits=(8, 6, 4), layers=
         for bi, b in enumerate(bits):
             try:
                 quantize_rows(w, [c], [b], write_back=True, want_codes=False)
-                values[ci * len(bits) + bi] = _evaluate(net, device, data_loader, want_probs=False)[1] - base
+                loss = _evaluate(net, device, data_loader, want_probs=False, shard=False)[1]
+                values[ci * len(bits) + bi] = loss - base
             except Exception as e:
                 flags[ci * len(bits) + bi] = 1.0
                 first_error = first_error or e

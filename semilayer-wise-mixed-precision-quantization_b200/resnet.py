@@ -181,6 +181,16 @@ class ResNet(nn.Module):
             self._slq_engines = {key: eng}  # one live shape at a time (activation buffers are large)
         return eng
 
+    def slq_calibrated(self, hw=None):
+        """True when a CUDA forward on images of size ``hw`` = (H, W) (None: of the size the net was calibrated at)
+        runs under activation scales the net already holds (its engine's, or through slq_share_calibration its
+        donor's); False when that forward calibrates them on its own batch (slq_engine() / forward())."""
+        eng = next(iter(self._slq_engines.values()), None)
+        donor = getattr(self, "_slq_donor", None)
+        if eng is None and donor is not None:
+            eng = next(iter(getattr(donor, "_slq_engines", {}).values()), None)
+        return eng is not None and eng.calibrated and (hw is None or eng.calib_hw == tuple(hw))
+
     def slq_share_calibration(self, other):
         """Use ``other``'s activation scales (same architecture, same image size) instead of calibrating on
         the first batch: the un-quantised model and the candidates of a sweep must be compared under the SAME
